@@ -25,6 +25,10 @@ all-gather of the capacity-constrained greedy).
 
 `--impl reference` times the reference's CPU implementation (the oracle port: no Go toolchain exists here,
 see DESIGN.md) with all host threads on a bounded sample of the same workload.
+
+`--steps K` is the number of timed steps of both timed passes (device and e2e).  `--dump-outputs DIR` writes, after
+them, what the last e2e step returned to its caller (pair records, per-server winners, decisions, per-type totals) as
+DIR/<name>.npy, so that two builds can be compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -241,6 +245,38 @@ def run_reference(args, rank, world):
     _emit(line)
 
 
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, per_server, per_pair, per_type, n_acc, limit=DUMP_LIMIT_BYTES, seed=0):
+    """Write every array as <out_dir>/<name>.npy: float32 data as float32, everything else as float64 (integers are
+    exact below 2^53).  per_pair arrays are server-major, n_acc entries per server.  When all files together would
+    exceed `limit` bytes, the per-server and per-pair arrays keep a fixed, seeded sample of the servers, whose indices
+    are written as sampled_servers.npy."""
+    def conv(d):
+        out = {}
+        for k, a in d.items():
+            a = np.asarray(a)
+            out[k] = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        return out
+
+    per_server, per_pair, out = conv(per_server), conv(per_pair), conv(per_type)
+    n_srv = len(next(iter(per_server.values())))
+    row = sum(a.itemsize for a in per_server.values()) + n_acc * sum(a.itemsize for a in per_pair.values())
+    budget = limit - sum(a.nbytes for a in out.values()) - 128 * (len(per_server) + len(per_pair) + len(out) + 1)  # .npy headers
+    if n_srv * row > budget:
+        srv = np.sort(np.random.default_rng(seed).choice(n_srv, max(0, budget // (row + 8)), replace=False))
+        pair = (srv[:, None] * n_acc + np.arange(n_acc)).ravel()
+        per_server = {k: a[srv] for k, a in per_server.items()}
+        per_pair = {k: a[pair] for k, a in per_pair.items()}
+        out["sampled_servers"] = srv.astype(np.float64)
+    out.update(per_server)
+    out.update(per_pair)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 _REAL_STDOUT = None
 
 
@@ -280,13 +316,20 @@ def main():
     ap.add_argument("--limited", action="store_true",
                     help="capacity-constrained assignment (SolveGreedy, PriorityExhaustive): capacities = 60 %% of the "
                          "unconstrained demand; multi-GPU ranks gather the candidate rows (one packed all-gather inside the library) and solve redundantly")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last e2e step returned (pair records, winners, decisions, per-type "
+                         "totals) as DIR/<name>.npy in float32 / float64, at most 64 MB (a fixed, seeded sample of the servers beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl == "reference" or world > 1):
+        ap.error("--dump-outputs writes the outputs of the CUDA path on one GPU (--impl ours, one rank)")
 
     if args.impl == "reference":
         run_reference(args, rank, world)
@@ -392,7 +435,7 @@ def main():
     value = cand_total / (ms_per_step * 1e-3)
 
     # ---- e2e through the public API (same work, host buffers) -----------------------------------
-    n_e2e = max(3, min(args.steps, 20))
+    n_e2e = args.steps
     for _ in range(2):
         out = step_e2e()
     barrier()
@@ -406,6 +449,13 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     e2e_s = float(t.item())
     pairs, best, chosen, tot = out
+    if args.dump_outputs:
+        per_server = {"winner_" + n: best[n] for n in best.dtype.names}
+        per_server["chosen_key"] = chosen[0]
+        per_server.update(("chosen_" + n, getattr(chosen[1], n)) for n, _ in abi.ALLOC_FIELDS)
+        per_pair = {"pairs_" + n: getattr(pairs[0], n) for n, _ in abi.ALLOC_FIELDS}
+        per_pair["pairs_feasible"] = pairs[1]
+        dump_outputs(args.dump_outputs, per_server, per_pair, {"type_count": tot[0], "type_cost": tot[1]}, img.A)
     h2d = img.nbytes()
     d2h = (sum(getattr(pairs[0], n).nbytes for n, _ in abi.ALLOC_FIELDS) + pairs[1].nbytes) * per_rank // img.S
     frac_dec = 1.0 if args.limited else per_rank / img.S            # a limited solve returns every server's decision on every rank
