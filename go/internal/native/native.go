@@ -197,6 +197,53 @@ func (c *Context) SetSweepFused(on bool) error {
 	return c.err(C.wva_grid_set_fused(c.ctx, v), "wva_grid_set_fused")
 }
 
+// SetSweepPairWinners: every later sweep (Analyze, AnalyzeGrid) also keeps its best candidate of each
+// (server, accelerator) pair on the device, for GridPairsFetch / SolveGrid.
+func (c *Context) SetSweepPairWinners(on bool) error {
+	c.mu.Lock()
+	defer c.mu.Unlock()
+	v := C.int32_t(0)
+	if on {
+		v = 1
+	}
+	return c.err(C.wva_grid_set_pair_winners(c.ctx, v), "wva_grid_set_pair_winners")
+}
+
+// GridPairsFetch copies the sweep's per-pair winners of the shard out: S*A records + feasible flags.
+func (c *Context) GridPairsFetch(s, a int) (*Allocs, []uint8, error) {
+	c.mu.Lock()
+	defer c.mu.Unlock()
+	n := s * a
+	if n == 0 {
+		return newAllocs(0), nil, nil
+	}
+	out, fe := newAllocs(n), make([]uint8, n)
+	rc := C.wva_grid_pairs_fetch_arrays(c.ctx, i32p(out.Acc), i64p(out.NumReplicas), i64p(out.BatchSize), f32p(out.Cost), f32p(out.Value),
+		f32p(out.ITL), f32p(out.TTFT), f32p(out.Rho), f32p(out.MaxArrv), u8p(fe))
+	if err := c.err(rc, "wva_grid_pairs_fetch_arrays"); err != nil {
+		return nil, nil, err
+	}
+	return out, fe, nil
+}
+
+// SolveGrid is Solve over the sweep's per-pair winners instead of the pair records.
+func (c *Context) SolveGrid(s int, unlimited, delayedBestEffort bool, policy int) ([]int32, *Allocs, int64, error) {
+	c.mu.Lock()
+	defer c.mu.Unlock()
+	b := func(v bool) C.int32_t { if v { return 1 }; return 0 }
+	if s == 0 {
+		return nil, newAllocs(0), 0, nil
+	}
+	key, out := make([]int32, s), newAllocs(s)
+	rc := C.wva_solve_grid_arrays(c.ctx, b(unlimited), b(delayedBestEffort), C.int32_t(policy), i32p(key),
+		i32p(out.Acc), i64p(out.NumReplicas), i64p(out.BatchSize), f32p(out.Cost), f32p(out.Value),
+		f32p(out.ITL), f32p(out.TTFT), f32p(out.Rho), f32p(out.MaxArrv))
+	if err := c.err(rc, "wva_solve_grid_arrays"); err != nil {
+		return nil, nil, 0, err
+	}
+	return key, out, int64(C.wva_solution_time_usec(c.ctx)), nil
+}
+
 // SetShard restricts the following calls to servers [first, first+count) (one process per GPU).
 func (c *Context) SetShard(first, count int) error {
 	c.mu.Lock()

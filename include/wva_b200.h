@@ -226,6 +226,12 @@ int wva_pairs_fetch_arrays(wva_ctx* ctx, int32_t* acc, int64_t* num_replicas, in
 int wva_solve_arrays(wva_ctx* ctx, int32_t unlimited, int32_t delayed_best_effort, int32_t saturation_policy,
         int32_t* chosen_acc, int32_t* acc, int64_t* num_replicas, int64_t* batch_size, float* cost, float* value,
         float* itl, float* ttft, float* rho, float* max_arrv_rate_per_replica);
+/* ... and of wva_grid_pairs_fetch / wva_solve_grid (sweep winners per pair, below) */
+int wva_grid_pairs_fetch_arrays(wva_ctx* ctx, int32_t* acc, int64_t* num_replicas, int64_t* batch_size, float* cost, float* value,
+        float* itl, float* ttft, float* rho, float* max_arrv_rate_per_replica, uint8_t* feasible);
+int wva_solve_grid_arrays(wva_ctx* ctx, int32_t unlimited, int32_t delayed_best_effort, int32_t saturation_policy,
+        int32_t* chosen_acc, int32_t* acc, int64_t* num_replicas, int64_t* batch_size, float* cost, float* value,
+        float* itl, float* ttft, float* rho, float* max_arrv_rate_per_replica);
 
 /* Multi-GPU sharding (SURVEY 8e): this rank owns servers [first, first+count) of the
  * uploaded image; analysis kernels touch only those; solve/allocate_by_type produce the
@@ -266,6 +272,32 @@ int wva_grid_fetch(wva_ctx* ctx, wva_grid_best* best);
  * wva_pairs_fetch / wva_grid_fetch copy them out, wva_solve consumes the pair records in place. */
 int wva_analyze(wva_ctx* ctx, int32_t r_max, int32_t b_max, int32_t want_cube);
 int wva_pairs_fetch(wva_ctx* ctx, wva_alloc_soa* out, uint8_t* feasible);
+
+/* Sweep winners per (server, accelerator) pair, as solver input.  With wva_grid_set_pair_winners(ctx, 1)
+ * (default 0) every sweep (wva_analyze_grid, wva_analyze_grid_device, wva_analyze, wva_group_analyze) also
+ * leaves S*A candidate records in HBM, laid out like the pair records of wva_analyze_pairs (a rank fills its
+ * shard rows).  The record of pair (s, a) is the sweep's feasible candidate of that pair with the smallest
+ * (value, replicas, batch) -- the per-server winner of wva_grid_best is the best of its pairs' records:
+ *     acc = a, num_replicas = r, batch_size = b,
+ *     cost  = acc.Cost * float32(numInstances * r), value = the transition penalty (as wva_grid_best),
+ *     itl, ttft, rho of the candidate (as wva_grid_best),
+ *     max_arrv_rate_per_replica = (totalRate / float32(r)) / 1000: the per-replica rate, req/msec, the candidate
+ *         was analysed at.  The sweep runs no QueueAnalyzer.Size, so this is NOT the SLO-bound rate that
+ *         CreateAllocation records there (allocation.go:141-160); the greedy does not read the field.
+ * feasible[s*A+a] = 0 (record empty, acc = WVA_ACC_NONE) when the pair has no feasible candidate: no load, not
+ * a candidate accelerator, or no (r, b) in the sweep's extents meets the SLOs.
+ * The records are invalidated by any image upload / update / shard change and by a sweep with the option off;
+ * a limited-capacity wva_solve_grid consumes them (best-effort scaling writes them in place).  They are
+ * independent of the pair records of wva_analyze_pairs.
+ *   wva_grid_pairs_fetch: copy the shard's records out (rows of other shards untouched), like wva_pairs_fetch;
+ *   wva_solve_grid: wva_solve (same unlimited argmin, same greedy paths, policies and delayed best-effort,
+ *       pkg/solver/solver.go:32-79, greedy.go:35-341) over the sweep records instead of the pair records.
+ *       It writes the same solution, so wva_allocate_by_type and wva_solution_time_usec work after it.  With a
+ *       communicator attached a limited solve all-gathers the records like wva_solve; without one it needs
+ *       the whole image as its shard.  WVA_ESTATE when no valid sweep records exist. */
+int wva_grid_set_pair_winners(wva_ctx* ctx, int32_t on);
+int wva_grid_pairs_fetch(wva_ctx* ctx, wva_alloc_soa* out, uint8_t* feasible);
+int wva_solve_grid(wva_ctx* ctx, const wva_optimizer_spec* spec, int32_t* chosen_acc, wva_alloc_soa* chosen);
 
 /* Device addresses of the S*A candidate records of wva_analyze_pairs (dev->... are DEVICE pointers,
  * server-major, same extents as the host variant).  Multi-GPU limited-capacity mode: each rank
@@ -399,6 +431,9 @@ int wva_group_analyze(wva_group* g, int32_t r_max, int32_t b_max, int32_t want_c
 int wva_group_pairs_fetch(wva_group* g, wva_alloc_soa* out, uint8_t* feasible);
 int wva_group_grid_fetch(wva_group* g, wva_grid_best* best /* [S] */);
 int wva_group_solve(wva_group* g, const wva_optimizer_spec* spec, int32_t* chosen_acc, wva_alloc_soa* chosen);
+/* the sweep-record forms (wva_grid_set_pair_winners on every device's ctx: wva_group_ctx) */
+int wva_group_grid_pairs_fetch(wva_group* g, wva_alloc_soa* out, uint8_t* feasible);
+int wva_group_solve_grid(wva_group* g, const wva_optimizer_spec* spec, int32_t* chosen_acc, wva_alloc_soa* chosen);
 int wva_group_allocate_by_type(wva_group* g, int64_t* count, float* cost);
 
 /* ---- low-level analyzer API (pkg/analyzer public surface) ------------------ */

@@ -29,6 +29,8 @@ EXPORTS = [
     "wva_comm_unique_id", "wva_comm_init", "wva_comm_destroy", "wva_comm_info", "wva_comm_shard",
     "wva_group_create", "wva_group_destroy", "wva_group_size", "wva_group_ctx", "wva_group_last_error", "wva_group_upload",
     "wva_group_analyze", "wva_group_pairs_fetch", "wva_group_grid_fetch", "wva_group_solve", "wva_group_allocate_by_type",
+    "wva_grid_set_pair_winners", "wva_grid_pairs_fetch", "wva_grid_pairs_fetch_arrays", "wva_solve_grid", "wva_solve_grid_arrays",
+    "wva_group_grid_pairs_fetch", "wva_group_solve_grid",
 ]
 
 
@@ -120,6 +122,11 @@ def lib():
         L.wva_group_grid_fetch.argtypes = [vp, vp]
         L.wva_group_solve.argtypes = [vp, C.POINTER(abi.OptimizerSpec), abi.i32p, C.POINTER(abi.AllocSoa)]
         L.wva_group_allocate_by_type.argtypes = [vp, abi.i64p, abi.f32p]
+        L.wva_grid_set_pair_winners.argtypes = [vp, i32]
+        L.wva_grid_pairs_fetch.argtypes = [vp, C.POINTER(abi.AllocSoa), abi.u8p]
+        L.wva_solve_grid.argtypes = [vp, C.POINTER(abi.OptimizerSpec), abi.i32p, C.POINTER(abi.AllocSoa)]
+        L.wva_group_grid_pairs_fetch.argtypes = [vp, C.POINTER(abi.AllocSoa), abi.u8p]
+        L.wva_group_solve_grid.argtypes = [vp, C.POINTER(abi.OptimizerSpec), abi.i32p, C.POINTER(abi.AllocSoa)]
         if L.wva_abi_version() != abi.ABI_VERSION:
             raise ImportError("libwva_b200.so ABI version mismatch")
         _lib = L
@@ -351,6 +358,18 @@ class Context:
     def grid_set_tail_cap(self, cap):
         self._ck(lib().wva_grid_set_tail_cap(self._h, int(cap)))
 
+    def grid_set_pair_winners(self, on):
+        """Every later sweep also keeps its best candidate of each (server, accelerator) pair on the device."""
+        self._ck(lib().wva_grid_set_pair_winners(self._h, 1 if on else 0))
+
+    def grid_pairs_fetch(self):
+        """The sweep's per-pair winners: (AllocArrays[S*A], feasible[S*A]); rows outside the shard are zero."""
+        n = self.image.S * self.image.A
+        out = abi.AllocArrays(n)
+        feasible = np.zeros(n, dtype=np.uint8)
+        self._ck(lib().wva_grid_pairs_fetch(self._h, C.byref(out.c), abi.ptr(feasible, C.c_uint8)))
+        return out, feasible
+
     def grid_list_sizes(self):
         a, b = C.c_int32(0), C.c_int32(0)
         self._ck(lib().wva_grid_list_sizes(self._h, C.byref(a), C.byref(b)))
@@ -384,6 +403,17 @@ class Context:
         chosen_acc = np.full(self.image.S, -1, dtype=np.int32)
         chosen = abi.AllocArrays(self.image.S)
         self._ck(lib().wva_solve(self._h, C.byref(spec), abi.ptr(chosen_acc, C.c_int32), C.byref(chosen.c)))
+        return chosen_acc, chosen
+
+    def solve_grid(self, unlimited=True, delayed_best_effort=False, policy=abi.POLICY_NONE, download=True):
+        """Solver.Solve over the sweep's per-pair winners.  Returns (chosen_acc[S], AllocArrays[S])."""
+        spec = abi.OptimizerSpec(1 if unlimited else 0, 1 if delayed_best_effort else 0, int(policy))
+        if not download:
+            self._ck(lib().wva_solve_grid(self._h, C.byref(spec), None, None))
+            return None
+        chosen_acc = np.full(self.image.S, -1, dtype=np.int32)
+        chosen = abi.AllocArrays(self.image.S)
+        self._ck(lib().wva_solve_grid(self._h, C.byref(spec), abi.ptr(chosen_acc, C.c_int32), C.byref(chosen.c)))
         return chosen_acc, chosen
 
     def allocate_by_type(self, download=True):
@@ -514,6 +544,27 @@ class Group:
         chosen_acc = np.full(self.image.S, -1, dtype=np.int32)
         chosen = abi.AllocArrays(self.image.S)
         self._ck(lib().wva_group_solve(self._h, C.byref(spec), abi.ptr(chosen_acc, C.c_int32), C.byref(chosen.c)))
+        return chosen_acc, chosen
+
+    def grid_set_pair_winners(self, on):
+        for c in self.ctxs:
+            c.grid_set_pair_winners(on)
+
+    def grid_pairs_fetch(self):
+        n = self.image.S * self.image.A
+        out = abi.AllocArrays(n)
+        feasible = np.zeros(n, dtype=np.uint8)
+        self._ck(lib().wva_group_grid_pairs_fetch(self._h, C.byref(out.c), abi.ptr(feasible, C.c_uint8)))
+        return out, feasible
+
+    def solve_grid(self, unlimited=True, delayed_best_effort=False, policy=abi.POLICY_NONE, download=True):
+        spec = abi.OptimizerSpec(1 if unlimited else 0, 1 if delayed_best_effort else 0, int(policy))
+        if not download:
+            self._ck(lib().wva_group_solve_grid(self._h, C.byref(spec), None, None))
+            return None
+        chosen_acc = np.full(self.image.S, -1, dtype=np.int32)
+        chosen = abi.AllocArrays(self.image.S)
+        self._ck(lib().wva_group_solve_grid(self._h, C.byref(spec), abi.ptr(chosen_acc, C.c_int32), C.byref(chosen.c)))
         return chosen_acc, chosen
 
     def allocate_by_type(self, download=True):

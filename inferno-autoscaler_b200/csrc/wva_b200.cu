@@ -211,6 +211,11 @@ struct wva_ctx {
     mutable bool pendS = false, pendT = false;
     int grid_r = 0, grid_b = 0; bool grid_valid = false;
     uint64_t grid_counters[3] = {0, 0, 0};
+    // per-(server, accelerator) sweep winners (wva_grid_set_pair_winners): full S*A extent like the pair records,
+    // a rank fills its shard rows; valid/complete as pairs_valid/pairs_complete
+    int grid_pair_winners = 0;
+    DevBuf gridPairBuf, gridPairKeys; DevAllocs gridPairs{}; unsigned char* gridFeasible = nullptr;
+    bool gpairs_valid = false, gpairs_complete = false;
 
     // multi-rank exchange (wva_comm_init / wva_group_create)
     nccl_comm_t comm = nullptr; int comm_rank = 0, comm_size = 1; bool comm_owned = false;
@@ -289,7 +294,7 @@ cudaError_t download_allocs(wva_ctx* ctx, const DevAllocs& d, size_t first, size
 
 // limited mode with a communicator: every rank packs the candidate records of its shard into one chunk,
 // ONE ncclAllGather moves all chunks, the other ranks' rows are scattered into place.
-int comm_gather_pairs(wva_ctx* ctx) {
+int comm_gather_pairs(wva_ctx* ctx, const DevAllocs& recs, unsigned char* feasible, bool& complete) {
     const NcclApi& nc = nccl_api();
     if (!nc.ok) return fail(ctx, WVA_ECUDA, "NCCL unavailable: " + nc.err);
     const int A = ctx->A, G = ctx->comm_size;
@@ -301,15 +306,15 @@ int comm_gather_pairs(wva_ctx* ctx) {
     CK(ctx->commChunk.ensure(chunkBytes));
     CK(ctx->commGather.ensure(chunkBytes * G));
     const int nPairs = ctx->ns * A;
-    k_pairs_pack<<<(nPairs + 255) / 256 + 1, 256, 0, ctx->stream>>>(ctx->pairs, ctx->feasible, ctx->s0 * A, nPairs, cap, ctx->commChunk.as<unsigned char>());
+    k_pairs_pack<<<(nPairs + 255) / 256 + 1, 256, 0, ctx->stream>>>(recs, feasible, ctx->s0 * A, nPairs, cap, ctx->commChunk.as<unsigned char>());
     LAUNCH_CHECK();
     int nrc = nc.AllGather(ctx->commChunk.p, ctx->commGather.p, chunkBytes, kNcclChar, ctx->comm, ctx->stream);
     if (nrc != 0) return fail(ctx, WVA_ECUDA, std::string("ncclAllGather(pairs): ") + nc.GetErrorString(nrc));
     dim3 grid((unsigned)((cap + 255) / 256 < 1024 ? (cap + 255) / 256 : 1024), (unsigned)G);
     k_pairs_unpack<<<grid, 256, 0, ctx->stream>>>(ctx->commGather.as<unsigned char>(), chunkBytes, cap, ctx->comm_rank, (size_t)ctx->S * A,
-                                                   ctx->pairs, ctx->feasible);
+                                                   recs, feasible);
     LAUNCH_CHECK();
-    ctx->pairs_complete = true;
+    complete = true;
     return WVA_OK;
 }
 
@@ -520,7 +525,7 @@ int wva_system_upload(wva_ctx* ctx, const wva_system_soa* h) {
     host_plan_rows(ctx, 0, S);
     ctx->plan_valid = false;
     ctx->have_system = true;
-    ctx->pairs_valid = ctx->pairs_complete = ctx->solved = ctx->grid_valid = false;
+    ctx->pairs_valid = ctx->pairs_complete = ctx->solved = ctx->grid_valid = ctx->gpairs_valid = ctx->gpairs_complete = false;
     timer.stop();
     return WVA_OK;
 }
@@ -531,7 +536,7 @@ int wva_set_shard(wva_ctx* ctx, int32_t first, int32_t count) {
     if (first < 0 || count < 0 || first + count > ctx->S) return fail(ctx, WVA_EINVAL, "shard out of range");
     ctx->s0 = first; ctx->ns = count;
     ctx->plan_valid = false;
-    ctx->pairs_valid = ctx->pairs_complete = ctx->solved = ctx->grid_valid = false;
+    ctx->pairs_valid = ctx->pairs_complete = ctx->solved = ctx->grid_valid = ctx->gpairs_valid = ctx->gpairs_complete = false;
     return WVA_OK;
 }
 
@@ -746,6 +751,7 @@ static int grid_run(wva_ctx* ctx, int r_max, int b_max, bool want_cube, bool wan
     if (r_max < 1 || r_max > WVA_GRID_MAX_R || b_max < 1 || b_max > WVA_GRID_MAX_B || ctx->A > WVA_GRID_MAX_A)
         return fail(ctx, WVA_EINVAL, "grid extents out of range (A<=256, r_max<=1024, b_max<=8192)");
     CK(cudaSetDevice(ctx->device));
+    ctx->gpairs_valid = ctx->gpairs_complete = false;
     const int ns = ctx->ns, A = ctx->A;
     const size_t nPairs = (size_t)ns * A;
     const size_t perPair = (size_t)r_max * (size_t)b_max;
@@ -792,6 +798,13 @@ static int grid_run(wva_ctx* ctx, int r_max, int b_max, bool want_cube, bool wan
     gp.status = want_status ? ctx->status.as<unsigned char>() : nullptr;
     gp.keys = ctx->keys.as<unsigned long long>();
     gp.counters = ctx->counters.as<unsigned long long>();
+    gp.pair_keys = nullptr; gp.pair_rec = DevAllocs{}; gp.pair_feasible = nullptr;
+    if (ctx->grid_pair_winners) {
+        const size_t nAll = (size_t)ctx->S * A;
+        CK(carve_allocs(ctx->gridPairBuf, nAll ? nAll : 1, ctx->gridPairs, &ctx->gridFeasible, nullptr));
+        CK(ctx->gridPairKeys.ensure((nPairs ? nPairs : 1) * 8));
+        gp.pair_keys = ctx->gridPairKeys.as<unsigned long long>(); gp.pair_rec = ctx->gridPairs; gp.pair_feasible = ctx->gridFeasible;
+    }
     gp.pair_tab = ctx->pairTab.as<double2>();
     // with certified tails almost no chain runs a long exact tail any more: finishing the few that do
     // inside the sweep kernel is cheaper than a second kernel + host round trip (cap < 0 = automatic)
@@ -896,7 +909,7 @@ static int grid_run(wva_ctx* ctx, int r_max, int b_max, bool want_cube, bool wan
     CK(cudaMemsetAsync(ctx->keys.p, 0xff, (size_t)(ns ? ns : 1) * 8, ctx->gstream));
     CK(cudaMemsetAsync(ctx->counters.p, 0, 3 * 8, ctx->gstream));
     if (ns > 0) {
-        k_grid_best_init<<<(ns + 255) / 256, 256, 0, ctx->gstream>>>(ns, ctx->bestDev.as<wva_grid_best>());
+        k_grid_best_init<<<(ns + 255) / 256, 256, 0, ctx->gstream>>>(ns, ctx->bestDev.as<wva_grid_best>(), gp, A);
         LAUNCH_CHECK();
     }
     for (int sBeg = 0; sBeg < ns; sBeg += srvPerSlice) {
@@ -1069,11 +1082,11 @@ static int grid_run(wva_ctx* ctx, int r_max, int b_max, bool want_cube, bool wan
         // winners of the slice: the slot that carries a server's minimum key writes its record
         if (nBlocks > 0) {
             const size_t nSlots = scanMode ? 2 * nBlocks : nBlocks;       // k_scan_cert and k_scan_lean each publish one slot per block
-            k_grid_claim<<<(unsigned)((nSlots + 255) / 256), 256, 0, ctx->gstream>>>(gp, gp.block_slot, (int)nSlots, ctx->bestDev.as<wva_grid_best>());
+            k_grid_claim<<<(unsigned)((nSlots + 255) / 256), 256, 0, ctx->gstream>>>(ctx->dsys, gp, gp.block_slot, (int)nSlots, ctx->bestDev.as<wva_grid_best>());
             LAUNCH_CHECK();
         }
         if (listSlots > 0) {
-            k_grid_claim<<<(listSlots + 255) / 256, 256, 0, ctx->gstream>>>(gp, gp.list_slot, listSlots, ctx->bestDev.as<wva_grid_best>());
+            k_grid_claim<<<(listSlots + 255) / 256, 256, 0, ctx->gstream>>>(ctx->dsys, gp, gp.list_slot, listSlots, ctx->bestDev.as<wva_grid_best>());
             LAUNCH_CHECK();
         }
     }
@@ -1086,6 +1099,8 @@ static int grid_run(wva_ctx* ctx, int r_max, int b_max, bool want_cube, bool wan
         CK(cudaStreamWaitEvent(ctx->stream, ctx->evJoin, 0));
     }
     ctx->grid_r = r_max; ctx->grid_b = b_max; ctx->grid_valid = true;
+    ctx->gpairs_valid = ctx->grid_pair_winners != 0;
+    ctx->gpairs_complete = ctx->gpairs_valid && ctx->s0 == 0 && ctx->ns == ctx->S;
     return WVA_OK;
 }
 
@@ -1185,6 +1200,23 @@ int wva_grid_set_fused(wva_ctx* ctx, int32_t on) {
     return WVA_OK;
 }
 int wva_grid_last_fused(const wva_ctx* ctx) { return ctx ? ctx->last_fused : WVA_EINVAL; }
+int wva_grid_set_pair_winners(wva_ctx* ctx, int32_t on) {
+    if (!ctx) return WVA_EINVAL;
+    ctx->grid_pair_winners = on ? 1 : 0;
+    return WVA_OK;
+}
+int wva_grid_pairs_fetch(wva_ctx* ctx, wva_alloc_soa* out, uint8_t* feasible) {
+    if (!ctx) return WVA_EINVAL;
+    if (!ctx->gpairs_valid) return fail(ctx, WVA_ESTATE, "no valid sweep winners per pair (wva_grid_set_pair_winners off, no sweep since, or consumed by a limited solve)");
+    CK(cudaSetDevice(ctx->device));
+    const size_t nPairs = (size_t)ctx->ns * ctx->A, first = (size_t)ctx->s0 * ctx->A;
+    if (nPairs > 0) {
+        if (out) CK(download_allocs(ctx, ctx->gridPairs, first, nPairs, out, first));
+        if (feasible) CK(cudaMemcpyAsync(feasible + first, ctx->gridFeasible + first, nPairs, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    return WVA_OK;
+}
 int wva_grid_list_sizes(const wva_ctx* ctx, int32_t* deferred, int32_t* literal) {
     if (!ctx) return WVA_EINVAL;
     if (deferred) *deferred = ctx->last_heavy;
@@ -1211,9 +1243,13 @@ int wva_grid_counters(const wva_ctx* ctx, uint64_t* steps_executed, uint64_t* st
 }
 
 // ---------------------------------------------------------------------------------------------
-int wva_solve(wva_ctx* ctx, const wva_optimizer_spec* spec, int32_t* chosen_acc, wva_alloc_soa* chosen) {
-    if (!ctx || !spec) return fail(ctx, WVA_EINVAL, "null argument");
-    if (!ctx->pairs_valid) return fail(ctx, WVA_ESTATE, "wva_solve needs wva_analyze_pairs first");
+}  // extern "C"
+
+// Solver.Solve over one candidate record set (S*A records + feasible flags): the pair records of
+// wva_analyze_pairs (wva_solve) or the sweep's per-pair winners (wva_solve_grid).  `valid` / `complete` are the
+// set's state flags: a limited solve gathers missing rows (communicator attached) and consumes the set.
+static int solve_records(wva_ctx* ctx, const wva_optimizer_spec* spec, int32_t* chosen_acc, wva_alloc_soa* chosen,
+                         const DevAllocs& recs, unsigned char* feasible, bool& valid, bool& complete, const char* incomplete_msg) {
     CK(cudaSetDevice(ctx->device));
     const int S = ctx->S, A = ctx->A, T = ctx->T;
     CK(carve_allocs(ctx->chosenBuf, (size_t)(S ? S : 1), ctx->chosen, nullptr, &ctx->chosen_acc));
@@ -1223,17 +1259,16 @@ int wva_solve(wva_ctx* ctx, const wva_optimizer_spec* spec, int32_t* chosen_acc,
     if (spec->unlimited) {
         first = ctx->s0; count = ctx->ns;          // separable: a rank solves its own servers
         if (count > 0) {
-            k_solve_unlimited<<<(count + 127) / 128, 128, 0, ctx->stream>>>(ctx->dsys, first, count, ctx->pairs, ctx->feasible,
+            k_solve_unlimited<<<(count + 127) / 128, 128, 0, ctx->stream>>>(ctx->dsys, first, count, recs, feasible,
                                                                           ctx->chosen_acc, ctx->chosen);
             LAUNCH_CHECK();
         }
     } else {
-        if (!ctx->pairs_complete && ctx->comm) {
-            int rc = comm_gather_pairs(ctx);
+        if (!complete && ctx->comm) {
+            int rc = comm_gather_pairs(ctx, recs, feasible, complete);
             if (rc != WVA_OK) return rc;
         }
-        if (!ctx->pairs_complete)
-            return fail(ctx, WVA_ESTATE, "limited-capacity solve needs the candidates of every server (wva_comm_init, or gather them and wva_pairs_commit)");
+        if (!complete) return fail(ctx, WVA_ESTATE, incomplete_msg);
         // carve greedy buffers
         if (T > 256) return fail(ctx, WVA_EINVAL, "the device greedy solver holds at most 256 accelerator types");
         if ((unsigned long long)(S ? S : 1) * (unsigned long long)A >= (1ull << 31))
@@ -1292,7 +1327,7 @@ int wva_solve(wva_ctx* ctx, const wva_optimizer_spec* spec, int32_t* chosen_acc,
         CK(cudaMemsetAsync(g.stats, 0, 32, ctx->stream));
         CK(cudaMemsetAsync(chosenKey, 0xff, nS * 4, ctx->stream));
         if (S > 0) {
-            k_greedy_prepare<<<(S + 127) / 128, 128, 0, ctx->stream>>>(ctx->dsys, ctx->pairs, ctx->feasible, g);
+            k_greedy_prepare<<<(S + 127) / 128, 128, 0, ctx->stream>>>(ctx->dsys, recs, feasible, g);
             LAUNCH_CHECK();
             k_greedy_bucket_count<<<(S + 255) / 256, 256, 0, ctx->stream>>>(ctx->dsys, g);
             LAUNCH_CHECK();
@@ -1337,7 +1372,7 @@ int wva_solve(wva_ctx* ctx, const wva_optimizer_spec* spec, int32_t* chosen_acc,
                 const bool tickets = spec->saturation_policy == WVA_POLICY_ROUND_ROBIN || spec->saturation_policy == WVA_POLICY_PRIORITY_ROUND_ROBIN;
                 if (tickets) smem = std::min((size_t)kGreedySmem, smem + nS * (sizeof(GreedyTicket) + 4));
                 g.smemBytes = (int)smem;
-                k_greedy_scan<<<1, 32, smem, ctx->stream>>>(ctx->dsys, ctx->pairs, g, gsc, chosenKey, spec->delayed_best_effort ? 1 : 0,
+                k_greedy_scan<<<1, 32, smem, ctx->stream>>>(ctx->dsys, recs, g, gsc, chosenKey, spec->delayed_best_effort ? 1 : 0,
                                                            spec->saturation_policy);
             }
             else if (ctx->greedy_path == 2) {
@@ -1347,20 +1382,20 @@ int wva_solve(wva_ctx* ctx, const wva_optimizer_spec* spec, int32_t* chosen_acc,
                 const bool tickets = spec->saturation_policy == WVA_POLICY_ROUND_ROBIN || spec->saturation_policy == WVA_POLICY_PRIORITY_ROUND_ROBIN;
                 if (tickets) smem = std::min((size_t)kGreedySmem, smem + nS * (sizeof(GreedyTicket) + 4));
                 g.smemBytes = (int)smem;
-                k_greedy_solve_ranked<<<1, 32, smem, ctx->stream>>>(ctx->dsys, ctx->pairs, g, gr, chosenKey,
+                k_greedy_solve_ranked<<<1, 32, smem, ctx->stream>>>(ctx->dsys, recs, g, gr, chosenKey,
                                                                    spec->delayed_best_effort ? 1 : 0, spec->saturation_policy);
             }
             else
-                k_greedy_solve<<<1, 32, kGreedySmem, ctx->stream>>>(ctx->dsys, ctx->pairs, g, chosenKey, spec->delayed_best_effort ? 1 : 0,
+                k_greedy_solve<<<1, 32, kGreedySmem, ctx->stream>>>(ctx->dsys, recs, g, chosenKey, spec->delayed_best_effort ? 1 : 0,
                                                                    spec->saturation_policy);
             LAUNCH_CHECK();
             ctx->greedy_stats_dev = g.stats;
-            k_greedy_collect<<<(S + 127) / 128, 128, 0, ctx->stream>>>(ctx->dsys, ctx->pairs, g.order, chosenKey, ctx->chosen_acc, ctx->chosen);
+            k_greedy_collect<<<(S + 127) / 128, 128, 0, ctx->stream>>>(ctx->dsys, recs, g.order, chosenKey, ctx->chosen_acc, ctx->chosen);
             LAUNCH_CHECK();
         }
         // best-effort scaling mutated the candidate records in place (greedy.go:208-212): the
-        // device copy no longer equals Server.Calculate's output
-        ctx->pairs_valid = false;
+        // device copy no longer equals what the analysis produced
+        valid = false;
     }
     if (spec->unlimited && !chosen_acc && !chosen) {
         // nothing goes back to the host: leave the work queued (later calls use the same stream) and read the
@@ -1381,6 +1416,24 @@ int wva_solve(wva_ctx* ctx, const wva_optimizer_spec* spec, int32_t* chosen_acc,
         CK(cudaStreamSynchronize(ctx->stream));
     }
     return WVA_OK;
+}
+
+extern "C" {
+
+int wva_solve(wva_ctx* ctx, const wva_optimizer_spec* spec, int32_t* chosen_acc, wva_alloc_soa* chosen) {
+    if (!ctx || !spec) return fail(ctx, WVA_EINVAL, "null argument");
+    if (!ctx->pairs_valid) return fail(ctx, WVA_ESTATE, "wva_solve needs wva_analyze_pairs first");
+    return solve_records(ctx, spec, chosen_acc, chosen, ctx->pairs, ctx->feasible, ctx->pairs_valid, ctx->pairs_complete,
+                         "limited-capacity solve needs the candidates of every server (wva_comm_init, or gather them and wva_pairs_commit)");
+}
+
+int wva_solve_grid(wva_ctx* ctx, const wva_optimizer_spec* spec, int32_t* chosen_acc, wva_alloc_soa* chosen) {
+    if (!ctx || !spec) return fail(ctx, WVA_EINVAL, "null argument");
+    if (!ctx->gpairs_valid)
+        return fail(ctx, WVA_ESTATE, "wva_solve_grid needs a sweep with wva_grid_set_pair_winners on (records are invalidated by an image "
+                                     "change or a sweep with the option off, and consumed by a limited solve)");
+    return solve_records(ctx, spec, chosen_acc, chosen, ctx->gridPairs, ctx->gridFeasible, ctx->gpairs_valid, ctx->gpairs_complete,
+                         "limited-capacity solve needs the sweep winners of every server (wva_comm_init)");
 }
 
 int wva_solve_set_ranked(wva_ctx* ctx, int32_t on) {
@@ -1775,6 +1828,19 @@ int wva_group_solve(wva_group* g, const wva_optimizer_spec* spec, int32_t* chose
     });
 }
 
+int wva_group_grid_pairs_fetch(wva_group* g, wva_alloc_soa* out, uint8_t* feasible) {
+    if (!g) return WVA_EINVAL;
+    return g->each([&](int, wva_ctx* c) { return wva_grid_pairs_fetch(c, out, feasible); });   // each ctx writes its own rows
+}
+
+int wva_group_solve_grid(wva_group* g, const wva_optimizer_spec* spec, int32_t* chosen_acc, wva_alloc_soa* chosen) {
+    if (!g || !spec) return WVA_EINVAL;
+    return g->each([&](int i, wva_ctx* c) {
+        const bool mine = spec->unlimited || i == 0;
+        return wva_solve_grid(c, spec, mine ? chosen_acc : nullptr, mine ? chosen : nullptr);
+    });
+}
+
 int wva_group_allocate_by_type(wva_group* g, int64_t* count, float* cost) {
     if (!g) return WVA_EINVAL;
     return g->each([&](int i, wva_ctx* c) { return wva_allocate_by_type(c, i == 0 ? count : nullptr, i == 0 ? cost : nullptr); });
@@ -1836,6 +1902,21 @@ int wva_solve_arrays(wva_ctx* ctx, int32_t unlimited, int32_t delayed_best_effor
     return wva_solve(ctx, &spec, chosen_acc, &o);
 }
 
+int wva_grid_pairs_fetch_arrays(wva_ctx* ctx, int32_t* acc, int64_t* num_replicas, int64_t* batch_size, float* cost, float* value,
+        float* itl, float* ttft, float* rho, float* max_arrv_rate_per_replica, uint8_t* feasible) {
+    wva_alloc_soa o = make_alloc_soa(acc, num_replicas, batch_size, cost, value, itl, ttft, rho, max_arrv_rate_per_replica);
+    return wva_grid_pairs_fetch(ctx, &o, feasible);
+}
+
+int wva_solve_grid_arrays(wva_ctx* ctx, int32_t unlimited, int32_t delayed_best_effort, int32_t saturation_policy,
+        int32_t* chosen_acc, int32_t* acc, int64_t* num_replicas, int64_t* batch_size, float* cost, float* value,
+        float* itl, float* ttft, float* rho, float* max_arrv_rate_per_replica) {
+    wva_optimizer_spec spec;
+    spec.unlimited = unlimited; spec.delayed_best_effort = delayed_best_effort; spec.saturation_policy = saturation_policy;
+    wva_alloc_soa o = make_alloc_soa(acc, num_replicas, batch_size, cost, value, itl, ttft, rho, max_arrv_rate_per_replica);
+    return wva_solve_grid(ctx, &spec, chosen_acc, &o);
+}
+
 }  // extern "C"
 
 // ---------------------------------------------------------------------------------------------
@@ -1846,7 +1927,7 @@ void invalidate_after_update(wva_ctx* ctx) {
     ctx->s0 = 0; ctx->ns = ctx->S;
     ctx->dsys.S = ctx->S; ctx->dsys.M = ctx->M;
     ctx->plan_valid = false;
-    ctx->pairs_valid = ctx->pairs_complete = ctx->solved = ctx->grid_valid = false;
+    ctx->pairs_valid = ctx->pairs_complete = ctx->solved = ctx->grid_valid = ctx->gpairs_valid = ctx->gpairs_complete = false;
 }
 }  // namespace
 

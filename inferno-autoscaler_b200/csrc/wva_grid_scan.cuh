@@ -347,6 +347,7 @@ __device__ __forceinline__ void scan_block_reduce(const DevSystem& sys, const Gr
         sl_.cost = gs.accCost * (float)go_muli(gs.numInst, (long long)r);
         gp.block_slot[slot] = sl_;
         atomicMin(&gp.keys[k.sl], blockKey);
+        if (gp.pair_keys) atomicMin(&gp.pair_keys[gp.pair_base + (int)(blockIdx.x / (unsigned)gp.n_rchunks)], blockKey);   // a block covers one pair (index re-derived: no register live across the sweep)
     }
     if (threadIdx.x == 0) {
         atomicAdd(&gp.counters[0], sh_cnt[0]); atomicAdd(&gp.counters[1], sh_cnt[1]); atomicAdd(&gp.counters[2], sh_cnt[2]);

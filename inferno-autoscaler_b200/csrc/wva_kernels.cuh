@@ -4,7 +4,7 @@
 //   k_grid           candidate sweep: one thread per (server, accel, replicas, batch) candidate,
 //                    service-rate tables staged in shared memory, warp-shuffle + block argmin
 //   k_grid_list      deferred long chains / materialised-p[] chains, one thread per candidate
-//   k_grid_claim     per-server winners from the published (key, metrics) slots
+//   k_grid_claim     per-server (and, when asked for, per-pair) winners from the published (key, metrics) slots
 //   k_solve_unlimited / k_greedy_*   the assignment step
 //   k_totals         System.AllocateByType partial sums (input of the one NCCL allreduce)
 //   k_queue_analyze / k_queue_size   the pkg/analyzer public API, batched
@@ -613,6 +613,10 @@ struct GridParams {
     unsigned long long* heavy_list; float* heavy_cost; int* heavy_count; int heavy_cap;   // deferred (long) chains
     ScanRow* row_info;               // [slice pairs * r_max] k_scan_prep -> k_scan_cert / k_scan_lean
     float2* rate_tab;                // [slice pairs * b_max] {RateRange.Max, RateTargetTPS} of batch size b (k_scan_prep)
+    // per-(server, accelerator) winners (wva_grid_set_pair_winners); pair_keys == nullptr: off
+    unsigned long long* pair_keys;   // [ns*A] per-pair argmin key (initialised to ~0), shard-local pair index
+    DevAllocs pair_rec;              // [S*A] records written by k_grid_claim (rows of the shard)
+    unsigned char* pair_feasible;    // [S*A]
 };
 
 // order-preserving map float -> uint32 (ascending), -0 canonicalised by the caller
@@ -868,6 +872,7 @@ k_grid(DevSystem sys, GridParams gp) {
         sl_.cost = gs.accCost * (float)go_muli(gs.numInst, (long long)r);
         gp.block_slot[blockIdx.x] = sl_;
         atomicMin(&gp.keys[sl], blockKey);
+        if (gp.pair_keys) atomicMin(&gp.pair_keys[gp.pair_base + (int)(blockIdx.x / (unsigned)gp.n_rchunks)], blockKey);   // a block covers one pair (index re-derived: no register live across the sweep)
     }
     if (threadIdx.x == 0) {
         atomicAdd(&gp.counters[0], sh_cnt[0]); atomicAdd(&gp.counters[1], sh_cnt[1]); atomicAdd(&gp.counters[2], sh_cnt[2]);
@@ -1123,6 +1128,7 @@ k_grid_rows(DevSystem sys, GridParams gp) {
         sl_.cost = gs.accCost * (float)go_muli(gs.numInst, (long long)r);
         gp.block_slot[blockIdx.x] = sl_;
         atomicMin(&gp.keys[sl], blockKey);
+        if (gp.pair_keys) atomicMin(&gp.pair_keys[gp.pair_base + (int)(blockIdx.x / (unsigned)gp.n_bseg)], blockKey);   // a block covers one pair (index re-derived: no register live across the sweep)
     }
     if (threadIdx.x == 0) {
         atomicAdd(&gp.counters[0], sh_cnt[0]); atomicAdd(&gp.counters[1], sh_cnt[1]); atomicAdd(&gp.counters[2], sh_cnt[2]);
@@ -1491,6 +1497,7 @@ k_grid_wrow(DevSystem sys, GridParams gp) {
         sl_.cost = gs.accCost * (float)go_muli(gs.numInst, (long long)r);
         gp.block_slot[blockIdx.x] = sl_;
         atomicMin(&gp.keys[sl], blockKey);
+        if (gp.pair_keys) atomicMin(&gp.pair_keys[gp.pair_base + (int)(blockIdx.x / (unsigned)gp.n_rchunks)], blockKey);   // a block covers one pair (index re-derived: no register live across the sweep)
     }
     if (threadIdx.x == 0) {
         atomicAdd(&gp.counters[0], sh_cnt[0]); atomicAdd(&gp.counters[1], sh_cnt[1]); atomicAdd(&gp.counters[2], sh_cnt[2]);
@@ -1546,6 +1553,10 @@ __device__ __forceinline__ void grid_list_item(const DevSystem& sys, const GridP
                 slot.key = key; slot.itl = m.avg_token_time; slot.ttft = m.avg_wait_time + m.avg_prefill_time;
                 slot.rho = m.rho; slot.cost = gs.accCost * (float)go_muli(gs.numInst, (long long)r);
                 if (key < gp.keys[sl]) atomicMin(&gp.keys[sl], key);
+                if (gp.pair_keys) {          // pair index from (sl, a), live here anyway
+                    unsigned long long* pk = gp.pair_keys + (sl * sys.A + a);
+                    if (key < *pk) atomicMin(pk, key);
+                }
             }
             alg += 2ULL * (unsigned long long)(11 * b + 1);
             okc += 1;
@@ -1687,6 +1698,10 @@ k_grid_list_warp(DevSystem sys, GridParams gp, const unsigned long long* __restr
                     slot.key = key; slot.itl = m.avg_token_time; slot.ttft = m.avg_wait_time + m.avg_prefill_time;
                     slot.rho = m.rho; slot.cost = gs.accCost * (float)go_muli(gs.numInst, (long long)r);
                     if (key < gp.keys[sl]) atomicMin(&gp.keys[sl], key);
+                    if (gp.pair_keys) {          // pair index from (sl, a), live here anyway
+                        unsigned long long* pk = gp.pair_keys + (sl * sys.A + a);
+                        if (key < *pk) atomicMin(pk, key);
+                    }
                 }
                 alg += 2ULL * (unsigned long long)(11 * b + 1);
                 okc += 1;
@@ -1746,23 +1761,52 @@ __global__ void k_heavy_scatter_dev(const float* __restrict__ cost, const int* _
 
 // Per-server winners: keys[] holds the minimum key of every server; the slot that carries that key
 // (exactly one: keys are unique per candidate) writes the wva_grid_best record.  No re-evaluation.
-__global__ void k_grid_best_init(int ns, wva_grid_best* __restrict__ best) {
+// With per-pair winners on, the pair keys and records of the shard are reset here too (empty record, infeasible).
+__global__ void k_grid_best_init(int ns, wva_grid_best* __restrict__ best, GridParams gp, int A) {
     int sl = blockIdx.x * blockDim.x + threadIdx.x;
     if (sl >= ns) return;
     wva_grid_best out;
     out.acc = -1; out.replicas = 0; out.batch = 0; out.cost = out.value = out.itl = out.ttft = out.rho = 0.0f;
     best[sl] = out;
+    if (gp.pair_keys) {
+        for (int a = 0; a < A; ++a) {
+            const size_t pl = (size_t)sl * A + a, gi = (size_t)gp.s0 * A + pl;
+            gp.pair_keys[pl] = WVA_KEY_NONE;
+            store_alloc(gp.pair_rec, gi, empty_alloc());
+            gp.pair_feasible[gi] = 0;
+        }
+    }
 }
-__global__ void k_grid_claim(GridParams gp, const GridSlot* __restrict__ slots, int nSlots, wva_grid_best* __restrict__ best) {
+// A slot that carries its server's minimum key writes the wva_grid_best record; with per-pair winners on, a slot that
+// carries its pair's minimum key also writes that pair's candidate record (a server's winner is its best pair's winner).
+__global__ void k_grid_claim(DevSystem sys, GridParams gp, const GridSlot* __restrict__ slots, int nSlots, wva_grid_best* __restrict__ best) {
     int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= nSlots) return;
     const GridSlot sl_ = slots[t];
     if (sl_.key == WVA_KEY_NONE) return;
+    const int a = (int)((sl_.key >> 24) & 0xff), r = (int)((sl_.key >> 14) & 0x3ff) + 1, b = (int)(sl_.key & 0x3fff) + 1;
+    const float value = unsortable_f32((unsigned)(sl_.key >> 32));
+    if (gp.pair_keys) {
+        const size_t pl = (size_t)sl_.sl * sys.A + a;
+        if (gp.pair_keys[pl] == sl_.key) {
+            // the per-replica rate the candidate was analysed at: scan_row_ctx's lambda (load_grid_server's totalRate)
+            const int s = gp.s0 + sl_.sl;
+            const float sloTPS = sys.srv_slo_tps[s];
+            const float totalRate = (sloTPS == 0.0f) ? sys.srv_arrival_rpm[s] / 60.0f : sloTPS / (float)(long long)sys.srv_out_tokens[s];
+            AllocRec rec;
+            rec.acc = a; rec.numReplicas = r; rec.batchSize = b;
+            rec.cost = sl_.cost; rec.value = value; rec.itl = sl_.itl; rec.ttft = sl_.ttft; rec.rho = sl_.rho;
+            rec.maxArrv = (totalRate / (float)r) / 1000.0f;
+            const size_t gi = (size_t)gp.s0 * sys.A + pl;
+            store_alloc(gp.pair_rec, gi, rec);
+            gp.pair_feasible[gi] = 1;
+        }
+    }
     if (gp.keys[sl_.sl] != sl_.key) return;
     wva_grid_best out;
-    out.acc = (int)((sl_.key >> 24) & 0xff); out.replicas = (int)((sl_.key >> 14) & 0x3ff) + 1; out.batch = (int)(sl_.key & 0x3fff) + 1;
+    out.acc = a; out.replicas = r; out.batch = b;
     out.cost = sl_.cost;
-    out.value = unsortable_f32((unsigned)(sl_.key >> 32));
+    out.value = value;
     out.itl = sl_.itl; out.ttft = sl_.ttft; out.rho = sl_.rho;
     best[sl_.sl] = out;
 }

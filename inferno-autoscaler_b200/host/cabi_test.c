@@ -5,7 +5,8 @@
  *     its size, no packing pragmas): offsets are asserted so that a change of the header that would
  *     silently change the Go-side layout fails here;
  * (3) on a box with a B200: the *_arrays entry points (what go/internal/native calls -- no struct of
- *     pointers crosses the boundary) give the same bytes as the struct forms.
+ *     pointers crosses the boundary) give the same bytes as the struct forms, for the pair records and for
+ *     the sweep's per-pair winners (wva_grid_pairs_fetch, wva_solve_grid).
  * Exit code 0 = ok (prints "no device" and stops after (2) when CUDA is unavailable). */
 #include <stddef.h>
 #include <stdio.h>
@@ -83,7 +84,26 @@ int main(void) {
     CHECK(nfe > 0);
     int64_t cnt[T]; float cst[T];
     CHECK(wva_allocate_by_type(ctx, cnt, cst) == WVA_OK);
-    printf("cabi_test: ok (%d feasible pairs, type counts %lld %lld)\n", nfe, (long long)cnt[0], (long long)cnt[1]);
+
+    /* the sweep's per-pair winners: fetch and solve, arrays forms against struct forms */
+    CHECK(wva_grid_set_pair_winners(ctx, 1) == WVA_OK);
+    CHECK(wva_analyze_grid_device(ctx, 8, 32, 0) == WVA_OK);
+    int32_t gacc1[S * A]; int64_t grep1[S * A], gbat1[S * A]; float gf1[6][S * A]; uint8_t gfe1[S * A];
+    int32_t gacc2[S * A]; int64_t grep2[S * A], gbat2[S * A]; float gf2[6][S * A]; uint8_t gfe2[S * A];
+    CHECK(wva_grid_pairs_fetch_arrays(ctx, gacc1, grep1, gbat1, gf1[0], gf1[1], gf1[2], gf1[3], gf1[4], gf1[5], gfe1) == WVA_OK);
+    wva_alloc_soa g2 = {gacc2, grep2, gbat2, gf2[0], gf2[1], gf2[2], gf2[3], gf2[4], gf2[5]};
+    CHECK(wva_grid_pairs_fetch(ctx, &g2, gfe2) == WVA_OK);
+    CHECK(!memcmp(gacc1, gacc2, sizeof gacc1) && !memcmp(grep1, grep2, sizeof grep1) && !memcmp(gbat1, gbat2, sizeof gbat1));
+    CHECK(!memcmp(gf1, gf2, sizeof gf1) && !memcmp(gfe1, gfe2, sizeof gfe1));
+    int ngfe = 0; for (int i = 0; i < S * A; ++i) ngfe += gfe1[i];
+    CHECK(ngfe > 0);
+    CHECK(wva_solve_grid_arrays(ctx, 1, 0, WVA_POLICY_NONE, key1, cacc1, crep1, cbat1, cf1[0], cf1[1], cf1[2], cf1[3], cf1[4], cf1[5]) == WVA_OK);
+    CHECK(wva_solve_grid(ctx, &spec, key2, &c2) == WVA_OK);
+    CHECK(!memcmp(key1, key2, sizeof key1) && !memcmp(cacc1, cacc2, sizeof cacc1) && !memcmp(crep1, crep2, sizeof crep1) && !memcmp(cf1, cf2, sizeof cf1));
+    CHECK(wva_grid_set_pair_winners(ctx, 0) == WVA_OK);
+    CHECK(wva_analyze_grid_device(ctx, 8, 32, 0) == WVA_OK);
+    CHECK(wva_solve_grid(ctx, &spec, key2, &c2) == WVA_ESTATE);                 /* a sweep with the option off */
+    printf("cabi_test: ok (%d feasible pairs, %d feasible sweep pairs, type counts %lld %lld)\n", nfe, ngfe, (long long)cnt[0], (long long)cnt[1]);
     wva_ctx_destroy(ctx);
     return 0;
 }
