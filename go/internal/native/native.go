@@ -226,6 +226,23 @@ func (c *Context) GridPairsFetch(s, a int) (*Allocs, []uint8, error) {
 	return out, fe, nil
 }
 
+// GridPairsSize runs QueueAnalyzer.Size on the device for every sweep record of the shard at the record's own
+// batch size; a sized record's MaxArrv becomes the SLO-bound rate per replica.  Status per pair of the S*A
+// extent: 0 no record, 1 sized, 2 Size failed (record unchanged); rows of other shards stay 0.
+func (c *Context) GridPairsSize(s, a int) ([]uint8, error) {
+	c.mu.Lock()
+	defer c.mu.Unlock()
+	n := s * a
+	if n == 0 {
+		return nil, nil
+	}
+	st := make([]uint8, n)
+	if err := c.err(C.wva_grid_pairs_size(c.ctx, u8p(st)), "wva_grid_pairs_size"); err != nil {
+		return nil, err
+	}
+	return st, nil
+}
+
 // SolveGrid is Solve over the sweep's per-pair winners instead of the pair records.
 func (c *Context) SolveGrid(s int, unlimited, delayedBestEffort bool, policy int) ([]int32, *Allocs, int64, error) {
 	c.mu.Lock()
@@ -419,6 +436,21 @@ func (g *Group) Analyze(rMax, bMax int) error {
 	g.mu.Lock()
 	defer g.mu.Unlock()
 	return g.err(C.wva_group_analyze(g.g, C.int32_t(rMax), C.int32_t(bMax), 0), "wva_group_analyze")
+}
+
+// GridPairsSize: Context.GridPairsSize on every device (each sizes its shard), status of the full S*A extent.
+func (g *Group) GridPairsSize(s, a int) ([]uint8, error) {
+	g.mu.Lock()
+	defer g.mu.Unlock()
+	n := s * a
+	if n == 0 {
+		return nil, nil
+	}
+	st := make([]uint8, n)
+	if err := g.err(C.wva_group_grid_pairs_size(g.g, u8p(st)), "wva_group_grid_pairs_size"); err != nil {
+		return nil, err
+	}
+	return st, nil
 }
 
 // AllocateByType: global per-type totals (NCCL all-gather of the partials inside the library).

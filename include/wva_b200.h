@@ -299,6 +299,23 @@ int wva_grid_set_pair_winners(wva_ctx* ctx, int32_t on);
 int wva_grid_pairs_fetch(wva_ctx* ctx, wva_alloc_soa* out, uint8_t* feasible);
 int wva_solve_grid(wva_ctx* ctx, const wva_optimizer_spec* spec, int32_t* chosen_acc, wva_alloc_soa* chosen);
 
+/* QueueAnalyzer.Size for every sweep record of the shard, at the record's own batch size.  For each pair (s, a) of
+ * the shard with a valid record of batch size b, what CreateAllocation computes at allocation.go:81-131 with N = b:
+ *     analyzer.NewQueueAnalyzer({MaxBatchSize b, MaxQueueSize 10 b, alpha beta gamma delta of (model, a)}, {in, out})
+ *     .Size({TTFT, ITL, TPS of the server})                                           (queueanalyzer.go:185-255)
+ * When Size succeeds, the record's max_arrv_rate_per_replica becomes float32(metrics.Throughput / 1000) (req/msec, as
+ * allocation.go:131, :160), so that MaxRPM / Saturated (allocation.go:233, :254) and the analyzer response see the
+ * SLO-bound rate; no other field changes.
+ *   status[s*A+a] (host, may be NULL; rows of other shards untouched): 0 = no record, 1 = sized, 2 = Size returned an
+ *       error and the record keeps the rate it was analysed at (e.g. a per-replica rate below Size's lambdaMin leaves
+ *       the bisection no bracket, utils.go:26-70).  The record stays solver input: the greedy does not read the field.
+ * WVA_ESTATE when no valid sweep records exist (as wva_grid_pairs_fetch).  Sized records stay valid:
+ * wva_grid_pairs_fetch and wva_solve_grid (every mode; a limited solve still consumes them) carry the sized rate; with
+ * a communicator attached each rank sizes its shard rows and the limited solve's all-gather moves the sized rates.
+ * Shards up to wva_pairs_set_warp_max pairs take one warp per pair, larger ones one thread per record; same results.
+ * Timed under WVA_PHASE_GRID_SIZE.  Nothing changes unless this is called. */
+int wva_grid_pairs_size(wva_ctx* ctx, uint8_t* status /* [S*A] host, may be NULL */);
+
 /* Device addresses of the S*A candidate records of wva_analyze_pairs (dev->... are DEVICE pointers,
  * server-major, same extents as the host variant).  Multi-GPU limited-capacity mode: each rank
  * fills its shard rows, the host all-gathers the rows over NCCL in place, then calls
@@ -434,6 +451,7 @@ int wva_group_solve(wva_group* g, const wva_optimizer_spec* spec, int32_t* chose
 /* the sweep-record forms (wva_grid_set_pair_winners on every device's ctx: wva_group_ctx) */
 int wva_group_grid_pairs_fetch(wva_group* g, wva_alloc_soa* out, uint8_t* feasible);
 int wva_group_solve_grid(wva_group* g, const wva_optimizer_spec* spec, int32_t* chosen_acc, wva_alloc_soa* chosen);
+int wva_group_grid_pairs_size(wva_group* g, uint8_t* status /* [S*A] */);
 int wva_group_allocate_by_type(wva_group* g, int64_t* count, float* cost);
 
 /* ---- low-level analyzer API (pkg/analyzer public surface) ------------------ */
@@ -480,6 +498,7 @@ int64_t wva_phase_time_usec(const wva_ctx* ctx, int phase);
 #define WVA_PHASE_TOTALS 4
 #define WVA_PHASE_GRID_KERNEL 5   /* the sweep kernel alone (events right around its launch) */
 #define WVA_PHASE_GRID_HEAVY  6   /* ordering + processing of the deferred long chains */
+#define WVA_PHASE_GRID_SIZE   7   /* wva_grid_pairs_size */
 /* The cudaStream_t every call of this ctx is enqueued on (so a host can record its own events
  * on it or order other work after it). */
 void* wva_stream(const wva_ctx* ctx);

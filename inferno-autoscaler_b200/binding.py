@@ -31,6 +31,7 @@ EXPORTS = [
     "wva_group_analyze", "wva_group_pairs_fetch", "wva_group_grid_fetch", "wva_group_solve", "wva_group_allocate_by_type",
     "wva_grid_set_pair_winners", "wva_grid_pairs_fetch", "wva_grid_pairs_fetch_arrays", "wva_solve_grid", "wva_solve_grid_arrays",
     "wva_group_grid_pairs_fetch", "wva_group_solve_grid",
+    "wva_grid_pairs_size", "wva_group_grid_pairs_size",
 ]
 
 
@@ -127,10 +128,21 @@ def lib():
         L.wva_solve_grid.argtypes = [vp, C.POINTER(abi.OptimizerSpec), abi.i32p, C.POINTER(abi.AllocSoa)]
         L.wva_group_grid_pairs_fetch.argtypes = [vp, C.POINTER(abi.AllocSoa), abi.u8p]
         L.wva_group_solve_grid.argtypes = [vp, C.POINTER(abi.OptimizerSpec), abi.i32p, C.POINTER(abi.AllocSoa)]
+        L.wva_grid_pairs_size.argtypes = [vp, abi.u8p]
+        L.wva_group_grid_pairs_size.argtypes = [vp, abi.u8p]
         if L.wva_abi_version() != abi.ABI_VERSION:
             raise ImportError("libwva_b200.so ABI version mismatch")
         _lib = L
     return _lib
+
+
+def _status_buffer(status, n):
+    """a caller's uint8[n] status buffer (written in place), or a new zeroed one"""
+    if status is None:
+        return np.zeros(n, dtype=np.uint8)
+    if not isinstance(status, np.ndarray) or status.dtype != np.uint8 or status.shape != (n,) or not status.flags.c_contiguous:
+        raise ValueError("status must be a contiguous uint8 array of S*A = %d entries" % n)
+    return status
 
 
 def comm_unique_id():
@@ -370,6 +382,14 @@ class Context:
         self._ck(lib().wva_grid_pairs_fetch(self._h, C.byref(out.c), abi.ptr(feasible, C.c_uint8)))
         return out, feasible
 
+    def grid_pairs_size(self, status=None):
+        """QueueAnalyzer.Size for every sweep record of the shard at its own batch size: a sized record's
+        max_arrv_rate_per_replica becomes the SLO-bound rate.  Returns status[S*A] (0 no record, 1 sized,
+        2 Size failed, record unchanged); rows outside the shard keep what `status` held (zeros when None)."""
+        status = _status_buffer(status, self.image.S * self.image.A)
+        self._ck(lib().wva_grid_pairs_size(self._h, abi.ptr(status, C.c_uint8)))
+        return status
+
     def grid_list_sizes(self):
         a, b = C.c_int32(0), C.c_int32(0)
         self._ck(lib().wva_grid_list_sizes(self._h, C.byref(a), C.byref(b)))
@@ -556,6 +576,12 @@ class Group:
         feasible = np.zeros(n, dtype=np.uint8)
         self._ck(lib().wva_group_grid_pairs_fetch(self._h, C.byref(out.c), abi.ptr(feasible, C.c_uint8)))
         return out, feasible
+
+    def grid_pairs_size(self, status=None):
+        """Context.grid_pairs_size on every device (each sizes its shard); status has the full extent S*A"""
+        status = _status_buffer(status, self.image.S * self.image.A)
+        self._ck(lib().wva_group_grid_pairs_size(self._h, abi.ptr(status, C.c_uint8)))
+        return status
 
     def solve_grid(self, unlimited=True, delayed_best_effort=False, policy=abi.POLICY_NONE, download=True):
         spec = abi.OptimizerSpec(1 if unlimited else 0, 1 if delayed_best_effort else 0, int(policy))

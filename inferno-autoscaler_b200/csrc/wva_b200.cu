@@ -216,6 +216,7 @@ struct wva_ctx {
     int grid_pair_winners = 0;
     DevBuf gridPairBuf, gridPairKeys; DevAllocs gridPairs{}; unsigned char* gridFeasible = nullptr;
     bool gpairs_valid = false, gpairs_complete = false;
+    DevBuf sizeStatus, sizeList, sizeCount;   // wva_grid_pairs_size
 
     // multi-rank exchange (wva_comm_init / wva_group_create)
     nccl_comm_t comm = nullptr; int comm_rank = 0, comm_size = 1; bool comm_owned = false;
@@ -392,7 +393,8 @@ void wva_ctx_destroy(wva_ctx* ctx) {
                       &ctx->greedyBuf, &ctx->keys, &ctx->bestDev, &ctx->cube, &ctx->status, &ctx->counters,
                       &ctx->gridSlow, &ctx->gridSlowCount, &ctx->faultList, &ctx->faultCount, &ctx->heavyList, &ctx->heavyCost,
                       &ctx->heavyOrder, &ctx->heavyHist, &ctx->pairTab, &ctx->blockSlot, &ctx->listSlot, &ctx->gscratch, &ctx->rowInfo, &ctx->rateTab, &ctx->ioA, &ctx->ioB,
-                      &ctx->ioC, &ctx->ioD, &ctx->ioE, &ctx->ioF, &ctx->ioG, &ctx->commTotals, &ctx->commChunk, &ctx->commGather};
+                      &ctx->ioC, &ctx->ioD, &ctx->ioE, &ctx->ioF, &ctx->ioG, &ctx->commTotals, &ctx->commChunk, &ctx->commGather,
+                      &ctx->sizeStatus, &ctx->sizeList, &ctx->sizeCount};
     for (DevBuf* b : bufs) b->release();
     ctx->staging.release();
     cudaEventDestroy(ctx->ev0);
@@ -1602,6 +1604,89 @@ int wva_queue_size(wva_ctx* ctx, int32_t n, const wva_queue_config* cfg, const f
     return WVA_OK;
 }
 
+// QueueAnalyzer.Size for every sweep record of the shard (kernels: wva_kernels.cuh, k_grid_size_*).  The warp path
+// (shards up to wva_pairs_set_warp_max pairs) lists what it cannot finish; the listed records, or all of them on the
+// thread path, are sized by k_queue_size, including its materialised-p[] re-run.
+int wva_grid_pairs_size(wva_ctx* ctx, uint8_t* status) {
+    if (!ctx) return WVA_EINVAL;
+    if (!ctx->gpairs_valid)
+        return fail(ctx, WVA_ESTATE, "no valid sweep winners per pair to size (wva_grid_set_pair_winners off, no sweep since, or consumed by a limited solve)");
+    CK(cudaSetDevice(ctx->device));
+    const int A = ctx->A, nPairs = ctx->ns * A;
+    const int firstPair = ctx->s0 * A;
+    CK(ctx->sizeStatus.ensure((size_t)(nPairs ? nPairs : 1)));
+    CK(ctx->sizeList.ensure((size_t)(nPairs ? nPairs : 1) * 4));
+    CK(ctx->sizeCount.ensure(4));
+    PhaseTimer timer(ctx, WVA_PHASE_GRID_SIZE);
+    if (nPairs > 0) {
+        int* list = ctx->sizeList.as<int>();
+        unsigned char* st = ctx->sizeStatus.as<unsigned char>();
+        CK(cudaMemsetAsync(ctx->sizeCount.p, 0, 4, ctx->stream));
+        if (nPairs <= ctx->pairs_warp_max) {
+            // a record's b is at most the sweep's b_max: the table fits the warp's slice of up to 3072 entries (48 KB)
+            // unless b_max is larger; records above the slice are listed
+            const int smemEntries = ctx->grid_b < 3072 ? ctx->grid_b : 3072;
+            const int warpsPerBlock = WVA_PAIRS_WARP_THREADS / 32;
+            const size_t smemBytes = (size_t)smemEntries * 16 * warpsPerBlock;
+            if (smemBytes > 48 * 1024)
+                CK(cudaFuncSetAttribute(k_grid_size_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemBytes));
+            k_grid_size_warp<<<(nPairs + warpsPerBlock - 1) / warpsPerBlock, WVA_PAIRS_WARP_THREADS, smemBytes, ctx->stream>>>(
+                ctx->dsys, ctx->s0, nPairs, ctx->gridPairs, ctx->gridFeasible, st, list, ctx->sizeCount.as<int>(), smemEntries);
+        } else {
+            k_grid_size_list<<<(nPairs + 255) / 256, 256, 0, ctx->stream>>>(firstPair, nPairs, ctx->gridFeasible, st, list,
+                                                                           ctx->sizeCount.as<int>());
+        }
+        LAUNCH_CHECK();
+        int n = 0;
+        CK(cudaMemcpyAsync(&n, ctx->sizeCount.p, 4, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        if (n > 0) {
+            CK(ctx->ioA.ensure((size_t)n * sizeof(wva_queue_config)));
+            CK(ctx->ioB.ensure((size_t)n * 12));
+            CK(ctx->ioC.ensure((size_t)n * sizeof(wva_metrics)));
+            CK(ctx->ioD.ensure((size_t)n));
+            CK(ctx->ioE.ensure((size_t)n * 12));
+            CK(ctx->ioF.ensure((size_t)n * 12));
+            CK(ctx->faultList.ensure((size_t)n * 4));
+            CK(ctx->faultCount.ensure(4));
+            wva_queue_config* cfg = ctx->ioA.as<wva_queue_config>();
+            k_grid_size_gather<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->dsys, ctx->s0, list, n, ctx->gridPairs, cfg, ctx->ioB.as<float>());
+            LAUNCH_CHECK();
+            CK(cudaMemsetAsync(ctx->faultCount.p, 0, 4, ctx->stream));
+            k_queue_size<<<(n + 127) / 128, 128, 0, ctx->stream>>>(n, cfg, ctx->ioB.as<float>(), ctx->ioE.as<float>(), ctx->ioC.as<wva_metrics>(),
+                                                                  ctx->ioF.as<float>(), ctx->ioD.as<unsigned char>(), nullptr, nullptr, nullptr,
+                                                                  ctx->faultList.as<int>(), ctx->faultCount.as<int>());
+            LAUNCH_CHECK();
+            int nf = 0;
+            CK(cudaMemcpyAsync(&nf, ctx->faultCount.p, 4, cudaMemcpyDeviceToHost, ctx->stream));
+            CK(cudaStreamSynchronize(ctx->stream));
+            if (nf > 0) {
+                // overflow-rescale chains: the same records again with p[] materialised in HBM (as wva_queue_size)
+                std::vector<int> flist((size_t)nf);
+                std::vector<wva_queue_config> hcfg((size_t)n);
+                CK(cudaMemcpy(flist.data(), ctx->faultList.p, (size_t)nf * 4, cudaMemcpyDeviceToHost));
+                CK(cudaMemcpy(hcfg.data(), cfg, (size_t)n * sizeof(wva_queue_config), cudaMemcpyDeviceToHost));
+                int rc = queue_scratch(ctx, hcfg.data(), flist, ctx->scratchOff);
+                if (rc != WVA_OK) return rc;
+                CK(ctx->ioG.ensure((size_t)nf * 4));
+                CK(cudaMemcpyAsync(ctx->ioG.p, flist.data(), (size_t)nf * 4, cudaMemcpyHostToDevice, ctx->stream));
+                k_queue_size<<<(nf + 127) / 128, 128, 0, ctx->stream>>>(nf, cfg, ctx->ioB.as<float>(), ctx->ioE.as<float>(), ctx->ioC.as<wva_metrics>(),
+                                                                       ctx->ioF.as<float>(), ctx->ioD.as<unsigned char>(), ctx->scratch.as<double>(),
+                                                                       ctx->scratchOff.as<long long>(), ctx->ioG.as<int>(),
+                                                                       ctx->faultList.as<int>(), ctx->faultCount.as<int>());
+                LAUNCH_CHECK();
+            }
+            k_grid_size_scatter<<<(n + 127) / 128, 128, 0, ctx->stream>>>(firstPair, list, n, ctx->ioC.as<wva_metrics>(),
+                                                                         ctx->ioD.as<unsigned char>(), ctx->gridPairs, st);
+            LAUNCH_CHECK();
+        }
+        if (status) CK(cudaMemcpyAsync(status + firstPair, st, (size_t)nPairs, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    CK(cudaStreamSynchronize(ctx->stream));
+    timer.stop();
+    return WVA_OK;
+}
+
 // ---------------------------------------------------------------------------------------------
 // Device self-test of the hoisted division: compares div_hoisted(a, b, rcp_refined(b)) with a / b
 // on n operand pairs produced on the device from a counter-based generator; returns the number of
@@ -1831,6 +1916,10 @@ int wva_group_solve(wva_group* g, const wva_optimizer_spec* spec, int32_t* chose
 int wva_group_grid_pairs_fetch(wva_group* g, wva_alloc_soa* out, uint8_t* feasible) {
     if (!g) return WVA_EINVAL;
     return g->each([&](int, wva_ctx* c) { return wva_grid_pairs_fetch(c, out, feasible); });   // each ctx writes its own rows
+}
+int wva_group_grid_pairs_size(wva_group* g, uint8_t* status) {
+    if (!g) return WVA_EINVAL;
+    return g->each([&](int, wva_ctx* c) { return wva_grid_pairs_size(c, status); });            // each ctx sizes its own rows
 }
 
 int wva_group_solve_grid(wva_group* g, const wva_optimizer_spec* spec, int32_t* chosen_acc, wva_alloc_soa* chosen) {

@@ -5,6 +5,7 @@
 //                    service-rate tables staged in shared memory, warp-shuffle + block argmin
 //   k_grid_list      deferred long chains / materialised-p[] chains, one thread per candidate
 //   k_grid_claim     per-server (and, when asked for, per-pair) winners from the published (key, metrics) slots
+//   k_grid_size_*    QueueAnalyzer.Size of the sweep's per-pair records (wva_grid_pairs_size)
 //   k_solve_unlimited / k_greedy_*   the assignment step
 //   k_totals         System.AllocateByType partial sums (input of the one NCCL allreduce)
 //   k_queue_analyze / k_queue_size   the pkg/analyzer public API, batched
@@ -301,39 +302,40 @@ __device__ __forceinline__ SolveStats shfl_stats(const SolveStats& s, int src) {
 }
 
 #define WVA_PAIRS_WARP_THREADS 128
-__global__ void __launch_bounds__(WVA_PAIRS_WARP_THREADS)
-k_pairs_warp(DevSystem sys, int s0, int nPairs, const long long* __restrict__ tabOff, double2* tabs, DevAllocs out,
-             unsigned char* feasible, int* slow_list, int* slow_count, unsigned long long* step_counter,
-             int smemEntriesPerWarp, double* pbuf, long long pbufStrideK, unsigned long long* dbg) {
-    extern __shared__ __align__(16) unsigned char pairs_smem[];
-    const long long tStart = clock64();
-    int activeRounds = 0, totalRounds = 0, pendEvals = 0;
-    long long solveCycles = 0;
-    const int pid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;      // warp-uniform
-    const int lane = threadIdx.x & 31;
-    if (pid >= nPairs) return;
-    const int s = s0 + pid / sys.A, a = pid % sys.A;
-    const size_t gi = (size_t)s * sys.A + a;
-    unsigned long long steps = 0;
-    AllocRec rec = empty_alloc();
-    bool ok = false;          // CreateAllocation != nil
-    bool toSlow = false;      // needs the materialised path (whole pair re-done by k_pairs_literal)
-
-    // every lane runs the scalar part redundantly (uniform control flow)
+// Shared part of the warp-per-pair kernels: one (server, accelerator) pair on one warp, every lane running the scalar
+// part redundantly (uniform control flow).  BuildModel (queueanalyzer.go:99-131, the {rate, refined reciprocal} table
+// built cooperatively), the two speculative half-warp bisections of QueueAnalyzer.Size and its trailing
+// Analyze(requestRate) (:185-241) are common to both instantiations:
+//   kAlloc = true  (k_pairs_warp): core.CreateAllocation -- N from the image, replicas, and the second Analyze
+//                  (allocation.go:148) speculated beside the trailing one; `rec` is the allocation, `ok` = non-nil;
+//   kAlloc = false (k_grid_size_warp): Size alone at N = `batch`, MaxQueueSize 10 N; ok: rec.maxArrv = Throughput / 1000,
+//                  !ok: Size returned an error.  The caller has checked that the pair holds a sweep record.
+// toSlow: the pair needs the thread path (no table budget / larger than the shared-memory slice, a bad service-rate
+// table, or a chain that needs the materialised p[]).
+template <bool kAlloc>
+__device__ __forceinline__ void warp_pair_size(const DevSystem& sys, const int s, const int a, const int pid, const int lane,
+                                               const long long batch, const long long* __restrict__ tabOff, double2* tabs,
+                                               unsigned char* smem, const int smemEntriesPerWarp, double* pbuf,
+                                               const long long pbufStrideK, unsigned long long* step_counter, AllocRec& rec, bool& ok,
+                                               bool& toSlow, unsigned long long& steps, int& activeRounds, int& totalRounds,
+                                               int& pendEvals, long long& solveCycles) {
     do {
-        if (!is_candidate_accel(sys, s, a) || !pair_lookups_ok(sys, s, a)) break;
+        if (kAlloc && (!is_candidate_accel(sys, s, a) || !pair_lookups_ok(sys, s, a))) break;
         const float arrival = sys.srv_arrival_rpm[s];
         const long long inTok = sys.srv_in_tokens[s], outTok = sys.srv_out_tokens[s];
-        if (arrival == 0.0f || outTok == 0) { rec = zero_load_allocation(sys, s, a); ok = true; break; }
+        if (kAlloc && (arrival == 0.0f || outTok == 0)) { rec = zero_load_allocation(sys, s, a); ok = true; break; }
         const int m = sys.srv_model[s];
         const size_t pi = (size_t)m * sys.A + a;
         const long long Kt = outTok;
-        long long N;
-        if (sys.srv_max_batch[s] > 0) N = sys.srv_max_batch[s];
-        else { N = go_divi(go_muli(sys.perf_max_batch[pi], sys.perf_at_tokens[pi]), Kt); if (N < 1) N = 1; }
+        long long N = batch;
+        if (kAlloc) {
+            if (sys.srv_max_batch[s] > 0) N = sys.srv_max_batch[s];
+            else { N = go_divi(go_muli(sys.perf_max_batch[pi], sys.perf_at_tokens[pi]), Kt); if (N < 1) N = 1; }
+        }
         const long long maxQueue = go_muli(N, WVA_MAX_QUEUE_TO_BATCH_RATIO);
         if (!config_ok(N, maxQueue, inTok, Kt)) break;
-        if (tabOff[pid] < 0 || N > (1LL << 26)) { toSlow = true; break; }   // no table budget: thread kernel handles it
+        // no table budget / (sizing) larger than the shared-memory slice: a thread kernel handles the pair
+        if (kAlloc ? (tabOff[pid] < 0 || N > (1LL << 26)) : N > smemEntriesPerWarp) { toSlow = true; break; }
         WarpPair wp;
         ServiceParms sp; sp.alpha = sys.perf_alpha[pi]; sp.beta = sys.perf_beta[pi];
         sp.gamma = sys.perf_gamma[pi]; sp.delta = sys.perf_delta[pi];
@@ -342,8 +344,8 @@ k_pairs_warp(DevSystem sys, int s0, int nPairs, const long long* __restrict__ ta
         wp.tame = tame_parms(sp, inTok, Kt);
         wp.cert = sys.cert != 0;
         // the table lives in shared memory when it fits (29-cycle loads in the ramp), else in HBM
-        double2* tab = (wp.N <= smemEntriesPerWarp)
-                           ? reinterpret_cast<double2*>(pairs_smem) + (size_t)(threadIdx.x >> 5) * smemEntriesPerWarp
+        double2* tab = (!kAlloc || wp.N <= smemEntriesPerWarp)
+                           ? reinterpret_cast<double2*>(smem) + (size_t)(threadIdx.x >> 5) * smemEntriesPerWarp
                            : tabs + tabOff[pid];
         wp.pstore = (pbuf && (long long)wp.K + 1 <= pbufStrideK) ? pbuf + (size_t)pid * (size_t)pbufStrideK * 32 + lane : nullptr;
         // BuildModel (queueanalyzer.go:99-131): the table, cooperatively
@@ -474,7 +476,7 @@ k_pairs_warp(DevSystem sys, int s0, int nPairs, const long long* __restrict__ ta
             }
             first = false;
         }
-        if (lane == 0) { atomicAdd(step_counter + 1, (unsigned long long)rounds); atomicMax(step_counter + 2, (unsigned long long)rounds); }
+        if (kAlloc && lane == 0) { atomicAdd(step_counter + 1, (unsigned long long)rounds); atomicMax(step_counter + 2, (unsigned long long)rounds); }
         if (toSlow) break;
         // results of the two bisections
         const bool failT = __shfl_sync(0xffffffffu, (int)failed, 0), failI = __shfl_sync(0xffffffffu, (int)failed, 16);
@@ -486,26 +488,30 @@ k_pairs_warp(DevSystem sys, int s0, int nPairs, const long long* __restrict__ ta
         if (tTPS > 0.0f) lTPS = lambdaMax * (1.0f - WVA_STABILITY_SAFETY);
         const float lambda = go_minf(go_minf(lTTFT, lITL), lTPS);
         const float requestRate = lambda * 1000.0f;
-        // ---- Analyze(requestRate) (:237-241) and Analyze(totalRate/replicas) (allocation.go:148) ----
+        // ---- Analyze(requestRate) (:237-241) and, kAlloc, Analyze(totalRate/replicas) (allocation.go:148) ----
         if (requestRate <= 0.0f || requestRate > wp.rateMax) break;        // :135-143 -> Size fails -> nil
         const float x1 = requestRate / 1000.0f;
-        float totalRate;
-        if (tTPS == 0.0f) totalRate = arrival / 60.0f;
-        else totalRate = tTPS / (float)Kt;
-        const int minRep = sys.srv_min_replicas[s];
-        // guess: throughput == x1 (blocking probability below float32 resolution)
-        const float rateStarGuess = x1 * 1000.0f;
-        long long repGuess = go_f64_to_int(ceil((double)totalRate / (double)rateStarGuess));
-        if (repGuess < (long long)minRep) repGuess = minRep;
-        const float rate2Guess = totalRate / (float)repGuess;
-        const bool rate2GuessOk = !(rate2Guess <= 0.0f) && !(rate2Guess > wp.rateMax);
+        float totalRate = 0.0f, rate2Guess = 0.0f;
+        int minRep = 0;
+        bool rate2GuessOk = false;
+        if (kAlloc) {
+            if (tTPS == 0.0f) totalRate = arrival / 60.0f;
+            else totalRate = tTPS / (float)Kt;
+            minRep = sys.srv_min_replicas[s];
+            // guess: throughput == x1 (blocking probability below float32 resolution)
+            const float rateStarGuess = x1 * 1000.0f;
+            long long repGuess = go_f64_to_int(ceil((double)totalRate / (double)rateStarGuess));
+            if (repGuess < (long long)minRep) repGuess = minRep;
+            rate2Guess = totalRate / (float)repGuess;
+            rate2GuessOk = !(rate2Guess <= 0.0f) && !(rate2Guess > wp.rateMax);
+        }
         // reuse an evaluation already made at exactly x1 if some lane has one
         const unsigned have = __ballot_sync(0xffffffffu, lastX == x1);
         SolveStats st1, st2;
         bool valid1 = true, valid2 = true, solved = true;
         {
             const bool needX1 = (have == 0u);
-            const bool actA = (lane == 0) && needX1, actB = (lane == 1) && rate2GuessOk;
+            const bool actA = (lane == 0) && needX1, actB = kAlloc && (lane == 1) && rate2GuessOk;
             SolveStats stl = st;
             bool v;
             bool uu;
@@ -518,6 +524,7 @@ k_pairs_warp(DevSystem sys, int s0, int nPairs, const long long* __restrict__ ta
         if (!valid1) break;
         wva_metrics m1; metrics_from(wp, st1, m1);
         const float rateStar = m1.throughput;
+        if (!kAlloc) { rec.maxArrv = rateStar / 1000.0f; ok = true; break; }    // Size's metrics.Throughput / 1000
         long long numReplicas = go_f64_to_int(ceil((double)totalRate / (double)rateStar));
         if (numReplicas < (long long)minRep) numReplicas = minRep;
         const long long totalNumInstances = go_muli(num_instances(sys, m, a), numReplicas);
@@ -542,6 +549,28 @@ k_pairs_warp(DevSystem sys, int s0, int nPairs, const long long* __restrict__ ta
         rec.value = cost;
         ok = true;
     } while (false);
+}
+
+__global__ void __launch_bounds__(WVA_PAIRS_WARP_THREADS)
+k_pairs_warp(DevSystem sys, int s0, int nPairs, const long long* __restrict__ tabOff, double2* tabs, DevAllocs out,
+             unsigned char* feasible, int* slow_list, int* slow_count, unsigned long long* step_counter,
+             int smemEntriesPerWarp, double* pbuf, long long pbufStrideK, unsigned long long* dbg) {
+    extern __shared__ __align__(16) unsigned char pairs_smem[];
+    const long long tStart = clock64();
+    int activeRounds = 0, totalRounds = 0, pendEvals = 0;
+    long long solveCycles = 0;
+    const int pid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;      // warp-uniform
+    const int lane = threadIdx.x & 31;
+    if (pid >= nPairs) return;
+    const int s = s0 + pid / sys.A, a = pid % sys.A;
+    const size_t gi = (size_t)s * sys.A + a;
+    unsigned long long steps = 0;
+    AllocRec rec = empty_alloc();
+    bool ok = false;          // CreateAllocation != nil
+    bool toSlow = false;      // needs the materialised path (whole pair re-done by k_pairs_literal)
+
+    warp_pair_size<true>(sys, s, a, pid, lane, 0, tabOff, tabs, pairs_smem, smemEntriesPerWarp, pbuf, pbufStrideK, step_counter,
+                         rec, ok, toSlow, steps, activeRounds, totalRounds, pendEvals, solveCycles);
 
     if (ok) rec.value = transition_penalty(sys.srv_cur_acc[s], sys.srv_cur_replicas[s], sys.srv_cur_cost[s], rec.acc,
                                            rec.numReplicas, rec.cost);
@@ -560,6 +589,73 @@ k_pairs_warp(DevSystem sys, int s0, int nPairs, const long long* __restrict__ ta
         feasible[gi] = ok ? 1 : 0;
         if (steps) atomicAdd(step_counter, steps);
     }
+}
+
+// ---------------------------------------------------------------------------------------
+// wva_grid_pairs_size: QueueAnalyzer.Size for every sweep record of the shard at the record's own batch size b
+// (CreateAllocation's Size, allocation.go:81-131, with N = b, MaxQueueSize = 10 b).  status[pid] (shard-local pair):
+// 0 no record, 1 sized (max_arrv_rate_per_replica = Throughput / 1000), 2 Size returned an error (record unchanged).
+// k_grid_size_warp (one warp per pair) lists the records it cannot finish; k_grid_size_list lists every record when
+// the thread path is chosen.  Listed records go through k_grid_size_gather -> k_queue_size -> k_grid_size_scatter.
+// ---------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(WVA_PAIRS_WARP_THREADS)
+k_grid_size_warp(DevSystem sys, int s0, int nPairs, DevAllocs recs, const unsigned char* __restrict__ feasible,
+                 unsigned char* __restrict__ status, int* list, int* list_count, int smemEntriesPerWarp) {
+    extern __shared__ __align__(16) unsigned char size_smem[];
+    const int pid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;      // warp-uniform
+    const int lane = threadIdx.x & 31;
+    if (pid >= nPairs) return;
+    const int s = s0 + pid / sys.A, a = pid % sys.A;
+    const size_t gi = (size_t)s * sys.A + a;
+    if (!feasible[gi]) { if (lane == 0) status[pid] = 0; return; }
+    unsigned long long steps = 0;
+    int activeRounds = 0, totalRounds = 0, pendEvals = 0;
+    long long solveCycles = 0;
+    AllocRec rec = empty_alloc();
+    bool ok = false, toSlow = false;
+    warp_pair_size<false>(sys, s, a, pid, lane, recs.batch_size[gi], nullptr, nullptr, size_smem, smemEntriesPerWarp, nullptr, 0,
+                          nullptr, rec, ok, toSlow, steps, activeRounds, totalRounds, pendEvals, solveCycles);
+    if (lane == 0) {
+        if (toSlow) list[atomicAdd(list_count, 1)] = pid;
+        else {
+            if (ok) recs.max_arrv[gi] = rec.maxArrv;
+            status[pid] = ok ? 1 : 2;
+        }
+    }
+}
+
+__global__ void k_grid_size_list(int firstPair, int nPairs, const unsigned char* __restrict__ feasible, unsigned char* __restrict__ status,
+                                 int* list, int* list_count) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= nPairs) return;
+    status[t] = 0;
+    if (feasible[(size_t)firstPair + t]) list[atomicAdd(list_count, 1)] = t;
+}
+
+// k_queue_size inputs of the listed records: {b, 10 b, alpha, beta, gamma, delta, in, out} and {TTFT, ITL, TPS}
+__global__ void k_grid_size_gather(DevSystem sys, int s0, const int* __restrict__ list, int n, DevAllocs recs,
+                                   wva_queue_config* __restrict__ cfg, float* __restrict__ target) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    const int pid = list[t];
+    const int s = s0 + pid / sys.A, a = pid % sys.A;
+    const size_t gi = (size_t)s * sys.A + a, pi = (size_t)sys.srv_model[s] * sys.A + a;
+    const long long b = recs.batch_size[gi];
+    wva_queue_config c;
+    c.max_batch_size = (int)b; c.max_queue_size = (int)go_muli(b, WVA_MAX_QUEUE_TO_BATCH_RATIO);
+    c.alpha = sys.perf_alpha[pi]; c.beta = sys.perf_beta[pi]; c.gamma = sys.perf_gamma[pi]; c.delta = sys.perf_delta[pi];
+    c.avg_input_tokens = sys.srv_in_tokens[s]; c.avg_output_tokens = sys.srv_out_tokens[s];
+    cfg[t] = c;
+    target[3 * t] = sys.srv_slo_ttft[s]; target[3 * t + 1] = sys.srv_slo_itl[s]; target[3 * t + 2] = sys.srv_slo_tps[s];
+}
+
+__global__ void k_grid_size_scatter(int firstPair, const int* __restrict__ list, int n, const wva_metrics* __restrict__ metrics,
+                                    const unsigned char* __restrict__ qstatus, DevAllocs recs, unsigned char* __restrict__ status) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    const int pid = list[t];
+    if (qstatus[t] == 0) recs.max_arrv[(size_t)firstPair + pid] = metrics[t].throughput / 1000.0f;
+    status[pid] = qstatus[t] == 0 ? 1 : 2;
 }
 
 // N per pair (0 = no queueing work) — used to order pairs by chain length and to size scratch.

@@ -6,7 +6,8 @@
  *     silently change the Go-side layout fails here;
  * (3) on a box with a B200: the *_arrays entry points (what go/internal/native calls -- no struct of
  *     pointers crosses the boundary) give the same bytes as the struct forms, for the pair records and for
- *     the sweep's per-pair winners (wva_grid_pairs_fetch, wva_solve_grid).
+ *     the sweep's per-pair winners (wva_grid_pairs_fetch, wva_solve_grid); wva_grid_pairs_size flags every
+ *     sweep record and nothing else.
  * Exit code 0 = ok (prints "no device" and stops after (2) when CUDA is unavailable). */
 #include <stddef.h>
 #include <stdio.h>
@@ -100,9 +101,15 @@ int main(void) {
     CHECK(wva_solve_grid_arrays(ctx, 1, 0, WVA_POLICY_NONE, key1, cacc1, crep1, cbat1, cf1[0], cf1[1], cf1[2], cf1[3], cf1[4], cf1[5]) == WVA_OK);
     CHECK(wva_solve_grid(ctx, &spec, key2, &c2) == WVA_OK);
     CHECK(!memcmp(key1, key2, sizeof key1) && !memcmp(cacc1, cacc2, sizeof cacc1) && !memcmp(crep1, crep2, sizeof crep1) && !memcmp(cf1, cf2, sizeof cf1));
+    /* Size on the records: a status byte for every record (1 sized / 2 Size failed), 0 where there is none */
+    uint8_t gst[S * A];
+    memset(gst, 0xee, sizeof gst);
+    CHECK(wva_grid_pairs_size(ctx, gst) == WVA_OK);
+    for (int i = 0; i < S * A; ++i) CHECK(gfe1[i] ? (gst[i] == 1 || gst[i] == 2) : gst[i] == 0);
     CHECK(wva_grid_set_pair_winners(ctx, 0) == WVA_OK);
     CHECK(wva_analyze_grid_device(ctx, 8, 32, 0) == WVA_OK);
     CHECK(wva_solve_grid(ctx, &spec, key2, &c2) == WVA_ESTATE);                 /* a sweep with the option off */
+    CHECK(wva_grid_pairs_size(ctx, gst) == WVA_ESTATE);
     printf("cabi_test: ok (%d feasible pairs, %d feasible sweep pairs, type counts %lld %lld)\n", nfe, ngfe, (long long)cnt[0], (long long)cnt[1]);
     wva_ctx_destroy(ctx);
     return 0;
