@@ -243,6 +243,45 @@ func (c *Context) GridPairsSize(s, a int) ([]uint8, error) {
 	return st, nil
 }
 
+// AnalyzeScenarios evaluates what Analyze -> unlimited Solve -> AllocateByType would give for every row of
+// arrivalRPM (nScen rows of s rates, row-major; each row replaces every server's arrival rate), one Size per pair.
+// Returns chosen[l*s+i] (-1 = none), the chosen records, and count / cost [l*t+j]; the resident image and results
+// are left untouched.
+func (c *Context) AnalyzeScenarios(s, t int, arrivalRPM []float32) ([]int32, *Allocs, []int64, []float32, error) {
+	c.mu.Lock()
+	defer c.mu.Unlock()
+	if s == 0 || len(arrivalRPM)%s != 0 {
+		return nil, nil, nil, nil, fmt.Errorf("AnalyzeScenarios: %d rates is not a whole number of %d-server rows", len(arrivalRPM), s)
+	}
+	l := len(arrivalRPM) / s
+	key, out := make([]int32, l*s), newAllocs(l*s)
+	count, cost := make([]int64, l*t), make([]float32, l*t)
+	rc := C.wva_analyze_scenarios_arrays(c.ctx, C.int32_t(l), f32p(arrivalRPM), i32p(key),
+		i32p(out.Acc), i64p(out.NumReplicas), i64p(out.BatchSize), f32p(out.Cost), f32p(out.Value),
+		f32p(out.ITL), f32p(out.TTFT), f32p(out.Rho), f32p(out.MaxArrv), i64p(count), f32p(cost))
+	if err := c.err(rc, "wva_analyze_scenarios_arrays"); err != nil {
+		return nil, nil, nil, nil, err
+	}
+	return key, out, count, cost, nil
+}
+
+// ScenarioPairsFetch copies scenario scen's S*A pair records of the last AnalyzeScenarios.
+func (c *Context) ScenarioPairsFetch(scen, s, a int) (*Allocs, []uint8, error) {
+	c.mu.Lock()
+	defer c.mu.Unlock()
+	n := s * a
+	if n == 0 {
+		return newAllocs(0), nil, nil
+	}
+	out, fe := newAllocs(n), make([]uint8, n)
+	rc := C.wva_scenario_pairs_fetch_arrays(c.ctx, C.int32_t(scen), i32p(out.Acc), i64p(out.NumReplicas), i64p(out.BatchSize),
+		f32p(out.Cost), f32p(out.Value), f32p(out.ITL), f32p(out.TTFT), f32p(out.Rho), f32p(out.MaxArrv), u8p(fe))
+	if err := c.err(rc, "wva_scenario_pairs_fetch_arrays"); err != nil {
+		return nil, nil, err
+	}
+	return out, fe, nil
+}
+
 // SolveGrid is Solve over the sweep's per-pair winners instead of the pair records.
 func (c *Context) SolveGrid(s int, unlimited, delayedBestEffort bool, policy int) ([]int32, *Allocs, int64, error) {
 	c.mu.Lock()

@@ -232,6 +232,12 @@ int wva_grid_pairs_fetch_arrays(wva_ctx* ctx, int32_t* acc, int64_t* num_replica
 int wva_solve_grid_arrays(wva_ctx* ctx, int32_t unlimited, int32_t delayed_best_effort, int32_t saturation_policy,
         int32_t* chosen_acc, int32_t* acc, int64_t* num_replicas, int64_t* batch_size, float* cost, float* value,
         float* itl, float* ttft, float* rho, float* max_arrv_rate_per_replica);
+/* ... and of wva_analyze_scenarios / wva_scenario_pairs_fetch (load scenarios, below) */
+int wva_analyze_scenarios_arrays(wva_ctx* ctx, int32_t n_scen, const float* arrival_rpm, int32_t* chosen_acc, int32_t* acc,
+        int64_t* num_replicas, int64_t* batch_size, float* cost, float* value, float* itl, float* ttft, float* rho,
+        float* max_arrv_rate_per_replica, int64_t* type_count, float* type_cost);
+int wva_scenario_pairs_fetch_arrays(wva_ctx* ctx, int32_t scen, int32_t* acc, int64_t* num_replicas, int64_t* batch_size, float* cost,
+        float* value, float* itl, float* ttft, float* rho, float* max_arrv_rate_per_replica, uint8_t* feasible);
 
 /* Multi-GPU sharding (SURVEY 8e): this rank owns servers [first, first+count) of the
  * uploaded image; analysis kernels touch only those; solve/allocate_by_type produce the
@@ -315,6 +321,37 @@ int wva_solve_grid(wva_ctx* ctx, const wva_optimizer_spec* spec, int32_t* chosen
  * Shards up to wva_pairs_set_warp_max pairs take one warp per pair, larger ones one thread per record; same results.
  * Timed under WVA_PHASE_GRID_SIZE.  Nothing changes unless this is called. */
 int wva_grid_pairs_size(wva_ctx* ctx, uint8_t* status /* [S*A] host, may be NULL */);
+
+/* What-if Analyze -> unlimited Optimize -> AllocateByType over n_scen load scenarios.  Scenario l replaces every
+ * server's ServerLoadSpec.ArrivalRate by arrival_rpm[l*S + s]; nothing else of the image changes.
+ *   Pair records: pair (s, a) of scenario l gets exactly what wva_analyze_pairs gives when the image's arrival rate of
+ *       s is arrival_rpm[l*S + s]: Server.Calculate's candidate filter, CreateAllocation and the transition penalty
+ *       (server.go:55-67, allocation.go:27-163, :291-300).  A negative rate gives nil (allocation.go:50), 0 gives
+ *       zeroLoadAllocation (:73-75).  Every input of QueueAnalyzer.Size is independent of the rate, so each pair runs
+ *       Size once and one trailing Analyze(totalRate / replicas) per scenario; a TPS-target server's positive
+ *       scenarios all share one (allocation.go:135-139).
+ *   chosen_acc[l*S + s], chosen[l*S + s] (host, may be NULL): SolveUnlimited of scenario l (solver.go:63-79), the
+ *       argmin of value with strict '<' from MaxFloat32 in ascending accelerator index, as wva_solve unlimited.
+ *   type_count[l*T + t], type_cost[l*T + t] (host, may be NULL): System.AllocateByType of scenario l
+ *       (system.go:271-300), summed in the fixed float32 order of wva_allocate_by_type.
+ * Limited-capacity (greedy) solves per scenario are not offered.
+ * The call leaves the image, the pair records, the sweep records, the solution and the totals as they were: a later
+ * wva_solve, wva_solve_grid or wva_allocate_by_type behaves as if it had not run.  Its records (L*S*A of 45 bytes,
+ * full S*A extent per scenario) stay valid for wva_scenario_pairs_fetch until the next wva_analyze_scenarios, image
+ * upload, image update or shard change; after those the fetch returns WVA_ESTATE.
+ * Errors: WVA_ESTATE without an uploaded image; WVA_EINVAL for n_scen outside [1, WVA_MAX_SCENARIOS] or a NaN / Inf
+ * rate; WVA_ECUDA when the record buffer cannot be allocated.
+ * With a communicator attached each rank fills its shard rows (records and chosen); the per-scenario partial totals
+ * {count[L*T]; cost[L*T]} move in ONE ncclAllGather and are summed in rank order (k_totals_merge over L*T entries), so
+ * every rank returns the global totals.  Shards up to wva_pairs_set_warp_max pairs take one warp per pair, larger
+ * ones one thread per pair and per (pair, scenario); same results.  The number of kernel launches does not grow with
+ * n_scen.  Timed under WVA_PHASE_SCENARIOS. */
+#define WVA_MAX_SCENARIOS 1024
+int wva_analyze_scenarios(wva_ctx* ctx, int32_t n_scen, const float* arrival_rpm /* [n_scen*S] host */,
+                          int32_t* chosen_acc /* [n_scen*S] or NULL */, wva_alloc_soa* chosen /* n_scen*S or NULL */,
+                          int64_t* type_count /* [n_scen*T] or NULL */, float* type_cost /* [n_scen*T] or NULL */);
+/* scenario scen's S*A records of the shard (rows of other shards untouched), like wva_pairs_fetch */
+int wva_scenario_pairs_fetch(wva_ctx* ctx, int32_t scen, wva_alloc_soa* out /* S*A */, uint8_t* feasible /* S*A */);
 
 /* Device addresses of the S*A candidate records of wva_analyze_pairs (dev->... are DEVICE pointers,
  * server-major, same extents as the host variant).  Multi-GPU limited-capacity mode: each rank
@@ -452,6 +489,10 @@ int wva_group_solve(wva_group* g, const wva_optimizer_spec* spec, int32_t* chose
 int wva_group_grid_pairs_fetch(wva_group* g, wva_alloc_soa* out, uint8_t* feasible);
 int wva_group_solve_grid(wva_group* g, const wva_optimizer_spec* spec, int32_t* chosen_acc, wva_alloc_soa* chosen);
 int wva_group_grid_pairs_size(wva_group* g, uint8_t* status /* [S*A] */);
+/* load scenarios: every device fills its shard rows of chosen_acc / chosen / the records; totals are global */
+int wva_group_analyze_scenarios(wva_group* g, int32_t n_scen, const float* arrival_rpm, int32_t* chosen_acc, wva_alloc_soa* chosen,
+                                int64_t* type_count, float* type_cost);
+int wva_group_scenario_pairs_fetch(wva_group* g, int32_t scen, wva_alloc_soa* out, uint8_t* feasible);
 int wva_group_allocate_by_type(wva_group* g, int64_t* count, float* cost);
 
 /* ---- low-level analyzer API (pkg/analyzer public surface) ------------------ */
@@ -499,6 +540,7 @@ int64_t wva_phase_time_usec(const wva_ctx* ctx, int phase);
 #define WVA_PHASE_GRID_KERNEL 5   /* the sweep kernel alone (events right around its launch) */
 #define WVA_PHASE_GRID_HEAVY  6   /* ordering + processing of the deferred long chains */
 #define WVA_PHASE_GRID_SIZE   7   /* wva_grid_pairs_size */
+#define WVA_PHASE_SCENARIOS   8   /* wva_analyze_scenarios (downloads excluded) */
 /* The cudaStream_t every call of this ctx is enqueued on (so a host can record its own events
  * on it or order other work after it). */
 void* wva_stream(const wva_ctx* ctx);

@@ -26,6 +26,8 @@ CAND_OK, CAND_FEASIBLE = 0, 1
 CAND_ERR_PAIR, CAND_ERR_CONFIG, CAND_ERR_RATE_LE0, CAND_ERR_RATE_MAX, CAND_ERR_MODEL = 2, 4, 6, 8, 10
 
 PHASE_UPLOAD, PHASE_PAIRS, PHASE_GRID, PHASE_SOLVE, PHASE_TOTALS, PHASE_GRID_KERNEL, PHASE_GRID_HEAVY, PHASE_GRID_SIZE = 0, 1, 2, 3, 4, 5, 6, 7
+PHASE_SCENARIOS = 8
+MAX_SCENARIOS = 1024
 
 MAX_QUEUE_TO_BATCH_RATIO = 10
 DEFAULT_PRIORITY = 100

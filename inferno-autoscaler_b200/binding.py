@@ -32,6 +32,8 @@ EXPORTS = [
     "wva_grid_set_pair_winners", "wva_grid_pairs_fetch", "wva_grid_pairs_fetch_arrays", "wva_solve_grid", "wva_solve_grid_arrays",
     "wva_group_grid_pairs_fetch", "wva_group_solve_grid",
     "wva_grid_pairs_size", "wva_group_grid_pairs_size",
+    "wva_analyze_scenarios", "wva_scenario_pairs_fetch", "wva_analyze_scenarios_arrays", "wva_scenario_pairs_fetch_arrays",
+    "wva_group_analyze_scenarios", "wva_group_scenario_pairs_fetch",
 ]
 
 
@@ -130,6 +132,10 @@ def lib():
         L.wva_group_solve_grid.argtypes = [vp, C.POINTER(abi.OptimizerSpec), abi.i32p, C.POINTER(abi.AllocSoa)]
         L.wva_grid_pairs_size.argtypes = [vp, abi.u8p]
         L.wva_group_grid_pairs_size.argtypes = [vp, abi.u8p]
+        L.wva_analyze_scenarios.argtypes = [vp, i32, abi.f32p, abi.i32p, C.POINTER(abi.AllocSoa), abi.i64p, abi.f32p]
+        L.wva_scenario_pairs_fetch.argtypes = [vp, i32, C.POINTER(abi.AllocSoa), abi.u8p]
+        L.wva_group_analyze_scenarios.argtypes = [vp, i32, abi.f32p, abi.i32p, C.POINTER(abi.AllocSoa), abi.i64p, abi.f32p]
+        L.wva_group_scenario_pairs_fetch.argtypes = [vp, i32, C.POINTER(abi.AllocSoa), abi.u8p]
         if L.wva_abi_version() != abi.ABI_VERSION:
             raise ImportError("libwva_b200.so ABI version mismatch")
         _lib = L
@@ -143,6 +149,29 @@ def _status_buffer(status, n):
     if not isinstance(status, np.ndarray) or status.dtype != np.uint8 or status.shape != (n,) or not status.flags.c_contiguous:
         raise ValueError("status must be a contiguous uint8 array of S*A = %d entries" % n)
     return status
+
+
+def _scenario_rates(arrival_rpm, S):
+    """the caller's [L, S] float32 scenario rates, checked before they reach the library"""
+    if not isinstance(arrival_rpm, np.ndarray) or arrival_rpm.dtype != np.float32:
+        raise TypeError("arrival_rpm must be a float32 numpy array of shape (n_scen, S)")
+    if arrival_rpm.ndim != 2 or arrival_rpm.shape[1] != S or not 1 <= arrival_rpm.shape[0] <= abi.MAX_SCENARIOS:
+        raise ValueError("arrival_rpm must have shape (n_scen, %d) with 1 <= n_scen <= %d, got %s"
+                         % (S, abi.MAX_SCENARIOS, arrival_rpm.shape))
+    if not np.isfinite(arrival_rpm).all():
+        raise ValueError("arrival_rpm holds NaN or Inf")
+    return np.ascontiguousarray(arrival_rpm)
+
+
+def _analyze_scenarios(fn, h, T, rates):
+    L, S = rates.shape
+    chosen_acc = np.full(L * S, -1, dtype=np.int32)
+    chosen = abi.AllocArrays(L * S)
+    count = np.zeros(L * T, dtype=np.int64)
+    cost = np.zeros(L * T, dtype=np.float32)
+    rc = fn(h, L, abi.ptr(rates, C.c_float), abi.ptr(chosen_acc, C.c_int32), C.byref(chosen.c), abi.ptr(count, C.c_int64),
+            abi.ptr(cost, C.c_float))
+    return rc, (chosen_acc.reshape(L, S), chosen, count.reshape(L, T), cost.reshape(L, T))
 
 
 def comm_unique_id():
@@ -390,6 +419,24 @@ class Context:
         self._ck(lib().wva_grid_pairs_size(self._h, abi.ptr(status, C.c_uint8)))
         return status
 
+    def analyze_scenarios(self, arrival_rpm):
+        """What-if Server.Calculate -> unlimited Solve -> AllocateByType for each row of arrival_rpm [L, S] (float32,
+        finite; row l replaces every server's arrival rate).  Returns (chosen_acc[L, S], AllocArrays[L*S],
+        count[L, T], cost[L, T]); rows of servers outside the shard stay -1 / zero.  The image, pair records,
+        solution and totals of the context are left untouched."""
+        rates = _scenario_rates(arrival_rpm, self.image.S)
+        rc, out = _analyze_scenarios(lib().wva_analyze_scenarios, self._h, self.image.T, rates)
+        self._ck(rc)
+        return out
+
+    def scenario_pairs_fetch(self, scen):
+        """Scenario scen's pair records: (AllocArrays[S*A], feasible[S*A]); rows outside the shard are zero."""
+        n = self.image.S * self.image.A
+        out = abi.AllocArrays(n)
+        feasible = np.zeros(n, dtype=np.uint8)
+        self._ck(lib().wva_scenario_pairs_fetch(self._h, int(scen), C.byref(out.c), abi.ptr(feasible, C.c_uint8)))
+        return out, feasible
+
     def grid_list_sizes(self):
         a, b = C.c_int32(0), C.c_int32(0)
         self._ck(lib().wva_grid_list_sizes(self._h, C.byref(a), C.byref(b)))
@@ -582,6 +629,20 @@ class Group:
         status = _status_buffer(status, self.image.S * self.image.A)
         self._ck(lib().wva_group_grid_pairs_size(self._h, abi.ptr(status, C.c_uint8)))
         return status
+
+    def analyze_scenarios(self, arrival_rpm):
+        """Context.analyze_scenarios on every device (each its shard); outputs have the full extent, totals are global"""
+        rates = _scenario_rates(arrival_rpm, self.image.S)
+        rc, out = _analyze_scenarios(lib().wva_group_analyze_scenarios, self._h, self.image.T, rates)
+        self._ck(rc)
+        return out
+
+    def scenario_pairs_fetch(self, scen):
+        n = self.image.S * self.image.A
+        out = abi.AllocArrays(n)
+        feasible = np.zeros(n, dtype=np.uint8)
+        self._ck(lib().wva_group_scenario_pairs_fetch(self._h, int(scen), C.byref(out.c), abi.ptr(feasible, C.c_uint8)))
+        return out, feasible
 
     def solve_grid(self, unlimited=True, delayed_best_effort=False, policy=abi.POLICY_NONE, download=True):
         spec = abi.OptimizerSpec(1 if unlimited else 0, 1 if delayed_best_effort else 0, int(policy))

@@ -6,6 +6,7 @@
 
 #include <atomic>
 #include <chrono>
+#include <cmath>
 #include <condition_variable>
 #include <cstdlib>
 #include <cstdio>
@@ -157,7 +158,7 @@ struct wva_ctx {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, evk0 = nullptr, evk1 = nullptr;
     std::string err;
     std::atomic<int64_t> launches{0};
-    int64_t phase_usec[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    int64_t phase_usec[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
 
     // system image: arrays are laid out with spare rows (Scap servers, Mcap models) so that the incremental
     // updates of pkg/core/system.go:99-171 touch only the rows that change (wva_system_update_*)
@@ -217,6 +218,11 @@ struct wva_ctx {
     DevBuf gridPairBuf, gridPairKeys; DevAllocs gridPairs{}; unsigned char* gridFeasible = nullptr;
     bool gpairs_valid = false, gpairs_complete = false;
     DevBuf sizeStatus, sizeList, sizeCount;   // wva_grid_pairs_size
+    // wva_analyze_scenarios: records of n_scen scenarios (full S*A extent each, a rank fills its shard rows), their
+    // unlimited solutions and totals; separate from everything above, which the call leaves untouched
+    DevBuf scenRates, scenRecBuf, scenChosenBuf, scenTotals, scenGather, scenList, scenCount, scenCfg, scenRate, scenMetrics, scenStatus;
+    DevAllocs scenPairs{}, scenChosen{}; unsigned char* scenFeasible = nullptr; int* scenChosenAcc = nullptr;
+    int scen_n = 0; bool scen_valid = false;
 
     // multi-rank exchange (wva_comm_init / wva_group_create)
     nccl_comm_t comm = nullptr; int comm_rank = 0, comm_size = 1; bool comm_owned = false;
@@ -267,7 +273,7 @@ cudaError_t carve_allocs(DevBuf& buf, size_t n, DevAllocs& a, unsigned char** fe
     auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
     size_t o_rep = take(n * 8), o_bat = take(n * 8), o_acc = take(n * 4), o_cost = take(n * 4), o_val = take(n * 4),
            o_itl = take(n * 4), o_ttft = take(n * 4), o_rho = take(n * 4), o_arr = take(n * 4), o_fe = take(n),
-           o_ch = take(n * 4);
+           o_ch = chosen_acc ? take(n * 4) : 0;
     cudaError_t e = buf.ensure(off);
     if (e != cudaSuccess) return e;
     char* b = buf.as<char>();
@@ -285,6 +291,22 @@ cudaError_t download_allocs(wva_ctx* ctx, const DevAllocs& d, size_t first, size
     if (h->field) {                                                                                                  \
         e = cudaMemcpyAsync(h->field + hfirst, d.dfield + first, n * sizeof(T), cudaMemcpyDeviceToHost, ctx->stream); \
         if (e != cudaSuccess) return e;                                                                              \
+    }
+    DL(acc, acc, int32_t) DL(num_replicas, num_replicas, int64_t) DL(batch_size, batch_size, int64_t)
+    DL(cost, cost, float) DL(value, value, float) DL(itl, itl, float) DL(ttft, ttft, float) DL(rho, rho, float)
+    DL(max_arrv_rate_per_replica, max_arrv, float)
+#undef DL
+    return cudaSuccess;
+}
+
+// rows [first, first + n) of each of `blocks` consecutive blocks of `pitch` records, into the same places of h
+cudaError_t download_allocs_blocks(wva_ctx* ctx, const DevAllocs& d, size_t first, size_t n, size_t pitch, size_t blocks, wva_alloc_soa* h) {
+    cudaError_t e;
+#define DL(field, dfield, T)                                                                                              \
+    if (h->field) {                                                                                                       \
+        e = cudaMemcpy2DAsync(h->field + first, pitch * sizeof(T), d.dfield + first, pitch * sizeof(T), n * sizeof(T), blocks, \
+                              cudaMemcpyDeviceToHost, ctx->stream);                                                       \
+        if (e != cudaSuccess) return e;                                                                                   \
     }
     DL(acc, acc, int32_t) DL(num_replicas, num_replicas, int64_t) DL(batch_size, batch_size, int64_t)
     DL(cost, cost, float) DL(value, value, float) DL(itl, itl, float) DL(ttft, ttft, float) DL(rho, rho, float)
@@ -394,7 +416,9 @@ void wva_ctx_destroy(wva_ctx* ctx) {
                       &ctx->gridSlow, &ctx->gridSlowCount, &ctx->faultList, &ctx->faultCount, &ctx->heavyList, &ctx->heavyCost,
                       &ctx->heavyOrder, &ctx->heavyHist, &ctx->pairTab, &ctx->blockSlot, &ctx->listSlot, &ctx->gscratch, &ctx->rowInfo, &ctx->rateTab, &ctx->ioA, &ctx->ioB,
                       &ctx->ioC, &ctx->ioD, &ctx->ioE, &ctx->ioF, &ctx->ioG, &ctx->commTotals, &ctx->commChunk, &ctx->commGather,
-                      &ctx->sizeStatus, &ctx->sizeList, &ctx->sizeCount};
+                      &ctx->sizeStatus, &ctx->sizeList, &ctx->sizeCount, &ctx->scenRates, &ctx->scenRecBuf, &ctx->scenChosenBuf,
+                      &ctx->scenTotals, &ctx->scenGather, &ctx->scenList, &ctx->scenCount, &ctx->scenCfg, &ctx->scenRate,
+                      &ctx->scenMetrics, &ctx->scenStatus};
     for (DevBuf* b : bufs) b->release();
     ctx->staging.release();
     cudaEventDestroy(ctx->ev0);
@@ -427,7 +451,7 @@ static void resolve_lazy_timers(const wva_ctx* ctx) {
     c->pendS = c->pendT = false;
 }
 int64_t wva_phase_time_usec(const wva_ctx* ctx, int phase) {
-    if (!ctx || phase < 0 || phase >= 8) return 0;
+    if (!ctx || phase < 0 || phase >= 9) return 0;
     resolve_lazy_timers(ctx);
     return ctx->phase_usec[phase];
 }
@@ -527,7 +551,7 @@ int wva_system_upload(wva_ctx* ctx, const wva_system_soa* h) {
     host_plan_rows(ctx, 0, S);
     ctx->plan_valid = false;
     ctx->have_system = true;
-    ctx->pairs_valid = ctx->pairs_complete = ctx->solved = ctx->grid_valid = ctx->gpairs_valid = ctx->gpairs_complete = false;
+    ctx->pairs_valid = ctx->pairs_complete = ctx->solved = ctx->grid_valid = ctx->gpairs_valid = ctx->gpairs_complete = ctx->scen_valid = false;
     timer.stop();
     return WVA_OK;
 }
@@ -538,7 +562,7 @@ int wva_set_shard(wva_ctx* ctx, int32_t first, int32_t count) {
     if (first < 0 || count < 0 || first + count > ctx->S) return fail(ctx, WVA_EINVAL, "shard out of range");
     ctx->s0 = first; ctx->ns = count;
     ctx->plan_valid = false;
-    ctx->pairs_valid = ctx->pairs_complete = ctx->solved = ctx->grid_valid = ctx->gpairs_valid = ctx->gpairs_complete = false;
+    ctx->pairs_valid = ctx->pairs_complete = ctx->solved = ctx->grid_valid = ctx->gpairs_valid = ctx->gpairs_complete = ctx->scen_valid = false;
     return WVA_OK;
 }
 
@@ -1262,7 +1286,7 @@ static int solve_records(wva_ctx* ctx, const wva_optimizer_spec* spec, int32_t* 
         first = ctx->s0; count = ctx->ns;          // separable: a rank solves its own servers
         if (count > 0) {
             k_solve_unlimited<<<(count + 127) / 128, 128, 0, ctx->stream>>>(ctx->dsys, first, count, recs, feasible,
-                                                                          ctx->chosen_acc, ctx->chosen);
+                                                                          ctx->chosen_acc, ctx->chosen, 0, 0);
             LAUNCH_CHECK();
         }
     } else {
@@ -1460,7 +1484,7 @@ int wva_allocate_by_type(wva_ctx* ctx, int64_t* count, float* cost) {
     ctx->pendT = false;
     long long* dcount = ctx->totals.as<long long>();
     float* dcost = (float*)(ctx->totals.as<char>() + (size_t)T * 8);
-    k_totals<<<T, 1024, 0, ctx->stream>>>(ctx->dsys, ctx->s0, ctx->ns, ctx->chosen_acc, ctx->chosen, dcount, dcost);
+    k_totals<<<T, 1024, 0, ctx->stream>>>(ctx->dsys, ctx->s0, ctx->ns, ctx->chosen_acc, ctx->chosen, dcount, dcost, 0);
     LAUNCH_CHECK();
     if (ctx->comm) {
         // the one exchange step of the path: all-gather of the {count, cost} partials, summed in rank order
@@ -1684,6 +1708,205 @@ int wva_grid_pairs_size(wva_ctx* ctx, uint8_t* status) {
     }
     CK(cudaStreamSynchronize(ctx->stream));
     timer.stop();
+    return WVA_OK;
+}
+
+}  // extern "C"
+
+// k_queue_size / k_queue_analyze listed rows in faultList (overflow-rescale chains): run them again with p[] materialised
+// in HBM, as wva_queue_size does.  `cfg` holds the n device rows the kernel read; relaunch(nf) issues the re-run over
+// the nf rows listed in ctx->ioG with the scratch offsets in ctx->scratchOff.
+template <class Relaunch>
+static int queue_fault_rerun(wva_ctx* ctx, const wva_queue_config* cfg, size_t n, Relaunch relaunch) {
+    int nf = 0;
+    CK(cudaMemcpyAsync(&nf, ctx->faultCount.p, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (nf == 0) return WVA_OK;
+    std::vector<int> flist((size_t)nf);
+    std::vector<wva_queue_config> hcfg(n);
+    CK(cudaMemcpy(flist.data(), ctx->faultList.p, (size_t)nf * 4, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(hcfg.data(), cfg, n * sizeof(wva_queue_config), cudaMemcpyDeviceToHost));
+    int rc = queue_scratch(ctx, hcfg.data(), flist, ctx->scratchOff);
+    if (rc != WVA_OK) return rc;
+    CK(ctx->ioG.ensure((size_t)nf * 4));
+    CK(cudaMemcpyAsync(ctx->ioG.p, flist.data(), (size_t)nf * 4, cudaMemcpyHostToDevice, ctx->stream));
+    relaunch(nf);
+    LAUNCH_CHECK();
+    return WVA_OK;
+}
+
+// wva_analyze_scenarios' thread path for n pairs (`list`, or every shard pair when list is null): one Size per pair
+// (k_queue_size), one Analyze per (pair, scenario) (k_queue_analyze), the records composed by k_scen_scatter
+static int scen_thread_path(wva_ctx* ctx, const int* list, int n, int L, const float* rates) {
+    const size_t rows = (size_t)n * L;
+    if (rows > 0x7fffffffULL) return fail(ctx, WVA_EINVAL, "pairs x scenarios on the thread path exceed 2^31-1 rows");
+    const int nr = (int)rows;
+    CK(ctx->ioA.ensure((size_t)n * sizeof(wva_queue_config)));
+    CK(ctx->ioB.ensure((size_t)n * 12));
+    CK(ctx->ioC.ensure((size_t)n * sizeof(wva_metrics)));
+    CK(ctx->ioD.ensure((size_t)n));
+    CK(ctx->ioE.ensure((size_t)n * 12));
+    CK(ctx->ioF.ensure((size_t)n * 12));
+    CK(ctx->scenCfg.ensure(rows * sizeof(wva_queue_config)));
+    CK(ctx->scenRate.ensure(rows * 4));
+    CK(ctx->scenMetrics.ensure(rows * sizeof(wva_metrics)));
+    CK(ctx->scenStatus.ensure(rows));
+    CK(ctx->faultList.ensure(rows * 4));
+    CK(ctx->faultCount.ensure(4));
+    wva_queue_config* cfg = ctx->ioA.as<wva_queue_config>();
+    float* target = ctx->ioB.as<float>();
+    wva_metrics* qm = ctx->ioC.as<wva_metrics>();
+    unsigned char* qs = ctx->ioD.as<unsigned char>();
+    wva_queue_config* rcfg = ctx->scenCfg.as<wva_queue_config>();
+    float* rrate = ctx->scenRate.as<float>();
+    wva_metrics* am = ctx->scenMetrics.as<wva_metrics>();
+    unsigned char* as = ctx->scenStatus.as<unsigned char>();
+    k_scen_gather<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->dsys, ctx->s0, list, n, L, rates, cfg, target);
+    LAUNCH_CHECK();
+    CK(cudaMemsetAsync(ctx->faultCount.p, 0, 4, ctx->stream));
+    k_queue_size<<<(n + 127) / 128, 128, 0, ctx->stream>>>(n, cfg, target, ctx->ioE.as<float>(), qm, ctx->ioF.as<float>(), qs, nullptr,
+                                                          nullptr, nullptr, ctx->faultList.as<int>(), ctx->faultCount.as<int>());
+    LAUNCH_CHECK();
+    int rc = queue_fault_rerun(ctx, cfg, (size_t)n, [&](int nf) {
+        k_queue_size<<<(nf + 127) / 128, 128, 0, ctx->stream>>>(nf, cfg, target, ctx->ioE.as<float>(), qm, ctx->ioF.as<float>(), qs,
+                                                               ctx->scratch.as<double>(), ctx->scratchOff.as<long long>(),
+                                                               ctx->ioG.as<int>(), ctx->faultList.as<int>(), ctx->faultCount.as<int>());
+    });
+    if (rc != WVA_OK) return rc;
+    const unsigned rowBlocks = (unsigned)((rows + 255) / 256);
+    k_scen_rows<<<rowBlocks, 256, 0, ctx->stream>>>(ctx->dsys, ctx->s0, list, n, L, rates, cfg, qm, qs, rcfg, rrate);
+    LAUNCH_CHECK();
+    CK(cudaMemsetAsync(ctx->faultCount.p, 0, 4, ctx->stream));
+    k_queue_analyze<<<(nr + 127) / 128, 128, 0, ctx->stream>>>(nr, rcfg, rrate, am, as, nullptr, nullptr, nullptr, ctx->faultList.as<int>(),
+                                                              ctx->faultCount.as<int>());
+    LAUNCH_CHECK();
+    rc = queue_fault_rerun(ctx, rcfg, rows, [&](int nf) {
+        k_queue_analyze<<<(nf + 127) / 128, 128, 0, ctx->stream>>>(nf, rcfg, rrate, am, as, ctx->scratch.as<double>(),
+                                                                  ctx->scratchOff.as<long long>(), ctx->ioG.as<int>(),
+                                                                  ctx->faultList.as<int>(), ctx->faultCount.as<int>());
+    });
+    if (rc != WVA_OK) return rc;
+    k_scen_scatter<<<rowBlocks, 256, 0, ctx->stream>>>(ctx->dsys, ctx->s0, list, n, L, rates, cfg, qm, qs, am, as, ctx->scenPairs,
+                                                      ctx->scenFeasible);
+    LAUNCH_CHECK();
+    return WVA_OK;
+}
+
+extern "C" {
+
+// What-if Server.Calculate -> SolveUnlimited -> AllocateByType over n_scen load scenarios (kernels: wva_kernels.cuh,
+// k_scen_*).  Shards up to wva_pairs_set_warp_max pairs take one warp per pair (listing what it cannot finish), larger
+// ones the thread path.  Everything else of the context is left as it was.
+int wva_analyze_scenarios(wva_ctx* ctx, int32_t n_scen, const float* arrival_rpm, int32_t* chosen_acc, wva_alloc_soa* chosen,
+                          int64_t* type_count, float* type_cost) {
+    if (!ctx) return WVA_EINVAL;
+    if (!ctx->have_system) return fail(ctx, WVA_ESTATE, "no system uploaded");
+    if (n_scen < 1 || n_scen > WVA_MAX_SCENARIOS) return fail(ctx, WVA_EINVAL, "n_scen must be in [1, 1024]");
+    if (!arrival_rpm) return fail(ctx, WVA_EINVAL, "arrival_rpm is NULL");
+    const int S = ctx->S, A = ctx->A, T = ctx->T, L = n_scen;
+    for (size_t i = 0; i < (size_t)L * S; ++i)
+        if (!std::isfinite(arrival_rpm[i])) return fail(ctx, WVA_EINVAL, "scenario arrival rates must be finite");
+    CK(cudaSetDevice(ctx->device));
+    ctx->scen_valid = false;
+    const size_t SA = (size_t)S * A;
+    const int nPairs = ctx->ns * A;
+    CK(ctx->scenRates.ensure((size_t)L * (S ? S : 1) * 4));
+    CK(carve_allocs(ctx->scenRecBuf, (size_t)L * (SA ? SA : 1), ctx->scenPairs, &ctx->scenFeasible, nullptr));
+    CK(carve_allocs(ctx->scenChosenBuf, (size_t)L * (S ? S : 1), ctx->scenChosen, nullptr, &ctx->scenChosenAcc));
+    CK(ctx->scenTotals.ensure((size_t)L * T * 12));
+    CK(ctx->scenList.ensure((size_t)(nPairs ? nPairs : 1) * 4));
+    CK(ctx->scenCount.ensure(4));
+    PhaseTimer timer(ctx, WVA_PHASE_SCENARIOS);
+    float* rates = ctx->scenRates.as<float>();
+    if (S > 0) CK(cudaMemcpyAsync(rates, arrival_rpm, (size_t)L * S * 4, cudaMemcpyHostToDevice, ctx->stream));
+    if (nPairs > 0) {
+        int n = nPairs;
+        const int* list = nullptr;
+        if (nPairs <= ctx->pairs_warp_max) {
+            // the warp's table slice: the shard's largest N (host copy of the image), at most 3072 entries (48 KB);
+            // larger pairs are listed
+            long long maxN = 0;
+            for (int s = ctx->s0; s < ctx->s0 + ctx->ns; ++s) {
+                const long long outTok = ctx->h_srv_out[(size_t)s];
+                const int m = ctx->h_srv_model[(size_t)s];
+                if (outTok <= 0 || m < 0) continue;
+                for (int a = 0; a < A; ++a) {
+                    long long N = ctx->h_srv_mb[(size_t)s];
+                    if (N <= 0) {
+                        const size_t pi = (size_t)m * A + a;
+                        N = (long long)ctx->h_pmb[pi] * (long long)ctx->h_pat[pi] / outTok;
+                    }
+                    if (N > maxN) maxN = N;
+                }
+            }
+            const int smemEntries = (int)(maxN < 3072 ? (maxN < 1 ? 1 : maxN) : 3072);
+            const int warpsPerBlock = WVA_PAIRS_WARP_THREADS / 32;
+            const size_t smemBytes = (size_t)smemEntries * 16 * warpsPerBlock;
+            if (smemBytes > 48 * 1024)
+                CK(cudaFuncSetAttribute(k_scen_pairs_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemBytes));
+            CK(cudaMemsetAsync(ctx->scenCount.p, 0, 4, ctx->stream));
+            k_scen_pairs_warp<<<(nPairs + warpsPerBlock - 1) / warpsPerBlock, WVA_PAIRS_WARP_THREADS, smemBytes, ctx->stream>>>(
+                ctx->dsys, ctx->s0, nPairs, L, rates, ctx->scenPairs, ctx->scenFeasible, ctx->scenList.as<int>(), ctx->scenCount.as<int>(),
+                smemEntries);
+            LAUNCH_CHECK();
+            CK(cudaMemcpyAsync(&n, ctx->scenCount.p, 4, cudaMemcpyDeviceToHost, ctx->stream));
+            CK(cudaStreamSynchronize(ctx->stream));
+            list = ctx->scenList.as<int>();
+        }
+        if (n > 0) {
+            int rc = scen_thread_path(ctx, list, n, L, rates);
+            if (rc != WVA_OK) return rc;
+        }
+        // SolveUnlimited of every scenario over the shard's servers
+        k_solve_unlimited<<<dim3((unsigned)((ctx->ns + 127) / 128), (unsigned)L), 128, 0, ctx->stream>>>(
+            ctx->dsys, ctx->s0, ctx->ns, ctx->scenPairs, ctx->scenFeasible, ctx->scenChosenAcc, ctx->scenChosen, SA, (size_t)S);
+        LAUNCH_CHECK();
+    }
+    // AllocateByType of every scenario: partials {count[L*T]; cost[L*T]}, with a communicator ONE all-gather and the
+    // rank-order sum of k_totals_merge over L*T entries
+    long long* dcount = ctx->scenTotals.as<long long>();
+    float* dcost = (float*)(ctx->scenTotals.as<char>() + (size_t)L * T * 8);
+    k_totals<<<dim3((unsigned)T, (unsigned)L), 1024, 0, ctx->stream>>>(ctx->dsys, ctx->s0, ctx->ns, ctx->scenChosenAcc, ctx->scenChosen,
+                                                                      dcount, dcost, (size_t)S);
+    LAUNCH_CHECK();
+    if (ctx->comm) {
+        const NcclApi& nc = nccl_api();
+        CK(ctx->scenGather.ensure((size_t)ctx->comm_size * L * T * 12));
+        int nrc = nc.AllGather(ctx->scenTotals.p, ctx->scenGather.p, (size_t)L * T * 12, kNcclChar, ctx->comm, ctx->stream);
+        if (nrc != 0) return fail(ctx, WVA_ECUDA, std::string("ncclAllGather(scenario totals): ") + nc.GetErrorString(nrc));
+        k_totals_merge<<<(L * T + 63) / 64, 64, 0, ctx->stream>>>(L * T, ctx->comm_size, ctx->scenGather.as<unsigned char>(), dcount, dcost);
+        LAUNCH_CHECK();
+    }
+    CK(cudaStreamSynchronize(ctx->stream));
+    timer.stop();
+    ctx->scen_n = L;
+    ctx->scen_valid = true;
+    if (ctx->ns > 0) {
+        const size_t first = (size_t)ctx->s0, cnt = (size_t)ctx->ns;
+        if (chosen_acc)
+            CK(cudaMemcpy2DAsync(chosen_acc + first, (size_t)S * 4, ctx->scenChosenAcc + first, (size_t)S * 4, cnt * 4, (size_t)L,
+                                 cudaMemcpyDeviceToHost, ctx->stream));
+        if (chosen) CK(download_allocs_blocks(ctx, ctx->scenChosen, first, cnt, (size_t)S, (size_t)L, chosen));
+    }
+    if (type_count) CK(cudaMemcpyAsync(type_count, dcount, (size_t)L * T * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    if (type_cost) CK(cudaMemcpyAsync(type_cost, dcost, (size_t)L * T * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return WVA_OK;
+}
+
+int wva_scenario_pairs_fetch(wva_ctx* ctx, int32_t scen, wva_alloc_soa* out, uint8_t* feasible) {
+    if (!ctx) return WVA_EINVAL;
+    if (!ctx->scen_valid)
+        return fail(ctx, WVA_ESTATE, "no scenario records (wva_analyze_scenarios has not run since the last image upload, update or shard change)");
+    if (scen < 0 || scen >= ctx->scen_n) return fail(ctx, WVA_EINVAL, "scenario index out of range");
+    CK(cudaSetDevice(ctx->device));
+    const size_t SA = (size_t)ctx->S * ctx->A, first = (size_t)ctx->s0 * ctx->A, n = (size_t)ctx->ns * ctx->A;
+    const size_t off = (size_t)scen * SA;
+    if (n > 0) {
+        if (out) CK(download_allocs(ctx, ctx->scenPairs, off + first, n, out, first));
+        if (feasible) CK(cudaMemcpyAsync(feasible + first, ctx->scenFeasible + off + first, n, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
     return WVA_OK;
 }
 
@@ -1922,6 +2145,19 @@ int wva_group_grid_pairs_size(wva_group* g, uint8_t* status) {
     return g->each([&](int, wva_ctx* c) { return wva_grid_pairs_size(c, status); });            // each ctx sizes its own rows
 }
 
+int wva_group_analyze_scenarios(wva_group* g, int32_t n_scen, const float* arrival_rpm, int32_t* chosen_acc, wva_alloc_soa* chosen,
+                                int64_t* type_count, float* type_cost) {
+    if (!g) return WVA_EINVAL;
+    // each ctx writes its own rows of chosen; the totals are global on every device -- device 0 returns them
+    return g->each([&](int i, wva_ctx* c) {
+        return wva_analyze_scenarios(c, n_scen, arrival_rpm, chosen_acc, chosen, i == 0 ? type_count : nullptr, i == 0 ? type_cost : nullptr);
+    });
+}
+int wva_group_scenario_pairs_fetch(wva_group* g, int32_t scen, wva_alloc_soa* out, uint8_t* feasible) {
+    if (!g) return WVA_EINVAL;
+    return g->each([&](int, wva_ctx* c) { return wva_scenario_pairs_fetch(c, scen, out, feasible); });   // each ctx writes its own rows
+}
+
 int wva_group_solve_grid(wva_group* g, const wva_optimizer_spec* spec, int32_t* chosen_acc, wva_alloc_soa* chosen) {
     if (!g || !spec) return WVA_EINVAL;
     return g->each([&](int i, wva_ctx* c) {
@@ -2006,6 +2242,19 @@ int wva_solve_grid_arrays(wva_ctx* ctx, int32_t unlimited, int32_t delayed_best_
     return wva_solve_grid(ctx, &spec, chosen_acc, &o);
 }
 
+int wva_analyze_scenarios_arrays(wva_ctx* ctx, int32_t n_scen, const float* arrival_rpm, int32_t* chosen_acc, int32_t* acc,
+        int64_t* num_replicas, int64_t* batch_size, float* cost, float* value, float* itl, float* ttft, float* rho,
+        float* max_arrv_rate_per_replica, int64_t* type_count, float* type_cost) {
+    wva_alloc_soa o = make_alloc_soa(acc, num_replicas, batch_size, cost, value, itl, ttft, rho, max_arrv_rate_per_replica);
+    return wva_analyze_scenarios(ctx, n_scen, arrival_rpm, chosen_acc, &o, type_count, type_cost);
+}
+
+int wva_scenario_pairs_fetch_arrays(wva_ctx* ctx, int32_t scen, int32_t* acc, int64_t* num_replicas, int64_t* batch_size, float* cost,
+        float* value, float* itl, float* ttft, float* rho, float* max_arrv_rate_per_replica, uint8_t* feasible) {
+    wva_alloc_soa o = make_alloc_soa(acc, num_replicas, batch_size, cost, value, itl, ttft, rho, max_arrv_rate_per_replica);
+    return wva_scenario_pairs_fetch(ctx, scen, &o, feasible);
+}
+
 }  // extern "C"
 
 // ---------------------------------------------------------------------------------------------
@@ -2016,7 +2265,7 @@ void invalidate_after_update(wva_ctx* ctx) {
     ctx->s0 = 0; ctx->ns = ctx->S;
     ctx->dsys.S = ctx->S; ctx->dsys.M = ctx->M;
     ctx->plan_valid = false;
-    ctx->pairs_valid = ctx->pairs_complete = ctx->solved = ctx->grid_valid = ctx->gpairs_valid = ctx->gpairs_complete = false;
+    ctx->pairs_valid = ctx->pairs_complete = ctx->solved = ctx->grid_valid = ctx->gpairs_valid = ctx->gpairs_complete = ctx->scen_valid = false;
 }
 }  // namespace
 

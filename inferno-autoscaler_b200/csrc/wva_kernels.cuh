@@ -7,6 +7,7 @@
 //   k_grid_claim     per-server (and, when asked for, per-pair) winners from the published (key, metrics) slots
 //   k_grid_size_*    QueueAnalyzer.Size of the sweep's per-pair records (wva_grid_pairs_size)
 //   k_solve_unlimited / k_greedy_*   the assignment step
+//   k_scen_*         Server.Calculate under many load scenarios, one Size per pair (wva_analyze_scenarios)
 //   k_totals         System.AllocateByType partial sums (input of the one NCCL allreduce)
 //   k_queue_analyze / k_queue_size   the pkg/analyzer public API, batched
 #pragma once
@@ -305,20 +306,27 @@ __device__ __forceinline__ SolveStats shfl_stats(const SolveStats& s, int src) {
 // Shared part of the warp-per-pair kernels: one (server, accelerator) pair on one warp, every lane running the scalar
 // part redundantly (uniform control flow).  BuildModel (queueanalyzer.go:99-131, the {rate, refined reciprocal} table
 // built cooperatively), the two speculative half-warp bisections of QueueAnalyzer.Size and its trailing
-// Analyze(requestRate) (:185-241) are common to both instantiations:
-//   kAlloc = true  (k_pairs_warp): core.CreateAllocation -- N from the image, replicas, and the second Analyze
+// Analyze(requestRate) (:185-241) are common to all instantiations:
+//   PAIR_ALLOC (k_pairs_warp): core.CreateAllocation -- N from the image, replicas, and the second Analyze
 //                  (allocation.go:148) speculated beside the trailing one; `rec` is the allocation, `ok` = non-nil;
-//   kAlloc = false (k_grid_size_warp): Size alone at N = `batch`, MaxQueueSize 10 N; ok: rec.maxArrv = Throughput / 1000,
-//                  !ok: Size returned an error.  The caller has checked that the pair holds a sweep record.
+//   PAIR_SIZE  (k_grid_size_warp): Size alone at N = `batch`, MaxQueueSize 10 N; ok: rec.maxArrv = Throughput / 1000,
+//                  !ok: Size returned an error.  The caller has checked that the pair holds a sweep record;
+//   PAIR_SCEN  (k_scen_pairs_warp): Size alone at CreateAllocation's N (allocation.go:77-87); ok: *pmOut holds the
+//                  pair's model, its table left in the warp's shared-memory slice, and Size's rateStar, for the caller's
+//                  per-scenario Analyze calls.  The caller has run the rate-independent checks (candidate, lookups) and
+//                  made sure the server has output tokens and some positive scenario rate.
 // toSlow: the pair needs the thread path (no table budget / larger than the shared-memory slice, a bad service-rate
 // table, or a chain that needs the materialised p[]).
-template <bool kAlloc>
+enum PairMode { PAIR_ALLOC, PAIR_SIZE, PAIR_SCEN };
+struct PairModel { WarpPair wp; float rateStar; };
+template <int kMode>
 __device__ __forceinline__ void warp_pair_size(const DevSystem& sys, const int s, const int a, const int pid, const int lane,
                                                const long long batch, const long long* __restrict__ tabOff, double2* tabs,
                                                unsigned char* smem, const int smemEntriesPerWarp, double* pbuf,
                                                const long long pbufStrideK, unsigned long long* step_counter, AllocRec& rec, bool& ok,
                                                bool& toSlow, unsigned long long& steps, int& activeRounds, int& totalRounds,
-                                               int& pendEvals, long long& solveCycles) {
+                                               int& pendEvals, long long& solveCycles, PairModel* pmOut = nullptr) {
+    constexpr bool kAlloc = kMode == PAIR_ALLOC, kScen = kMode == PAIR_SCEN;
     do {
         if (kAlloc && (!is_candidate_accel(sys, s, a) || !pair_lookups_ok(sys, s, a))) break;
         const float arrival = sys.srv_arrival_rpm[s];
@@ -328,7 +336,7 @@ __device__ __forceinline__ void warp_pair_size(const DevSystem& sys, const int s
         const size_t pi = (size_t)m * sys.A + a;
         const long long Kt = outTok;
         long long N = batch;
-        if (kAlloc) {
+        if (kAlloc || kScen) {
             if (sys.srv_max_batch[s] > 0) N = sys.srv_max_batch[s];
             else { N = go_divi(go_muli(sys.perf_max_batch[pi], sys.perf_at_tokens[pi]), Kt); if (N < 1) N = 1; }
         }
@@ -524,6 +532,7 @@ __device__ __forceinline__ void warp_pair_size(const DevSystem& sys, const int s
         if (!valid1) break;
         wva_metrics m1; metrics_from(wp, st1, m1);
         const float rateStar = m1.throughput;
+        if (kScen) { pmOut->wp = wp; pmOut->wp.pv.sf = &pmOut->wp.sv; pmOut->rateStar = rateStar; ok = true; break; }
         if (!kAlloc) { rec.maxArrv = rateStar / 1000.0f; ok = true; break; }    // Size's metrics.Throughput / 1000
         long long numReplicas = go_f64_to_int(ceil((double)totalRate / (double)rateStar));
         if (numReplicas < (long long)minRep) numReplicas = minRep;
@@ -569,8 +578,8 @@ k_pairs_warp(DevSystem sys, int s0, int nPairs, const long long* __restrict__ ta
     bool ok = false;          // CreateAllocation != nil
     bool toSlow = false;      // needs the materialised path (whole pair re-done by k_pairs_literal)
 
-    warp_pair_size<true>(sys, s, a, pid, lane, 0, tabOff, tabs, pairs_smem, smemEntriesPerWarp, pbuf, pbufStrideK, step_counter,
-                         rec, ok, toSlow, steps, activeRounds, totalRounds, pendEvals, solveCycles);
+    warp_pair_size<PAIR_ALLOC>(sys, s, a, pid, lane, 0, tabOff, tabs, pairs_smem, smemEntriesPerWarp, pbuf, pbufStrideK, step_counter,
+                               rec, ok, toSlow, steps, activeRounds, totalRounds, pendEvals, solveCycles);
 
     if (ok) rec.value = transition_penalty(sys.srv_cur_acc[s], sys.srv_cur_replicas[s], sys.srv_cur_cost[s], rec.acc,
                                            rec.numReplicas, rec.cost);
@@ -613,8 +622,8 @@ k_grid_size_warp(DevSystem sys, int s0, int nPairs, DevAllocs recs, const unsign
     long long solveCycles = 0;
     AllocRec rec = empty_alloc();
     bool ok = false, toSlow = false;
-    warp_pair_size<false>(sys, s, a, pid, lane, recs.batch_size[gi], nullptr, nullptr, size_smem, smemEntriesPerWarp, nullptr, 0,
-                          nullptr, rec, ok, toSlow, steps, activeRounds, totalRounds, pendEvals, solveCycles);
+    warp_pair_size<PAIR_SIZE>(sys, s, a, pid, lane, recs.batch_size[gi], nullptr, nullptr, size_smem, smemEntriesPerWarp, nullptr, 0,
+                              nullptr, rec, ok, toSlow, steps, activeRounds, totalRounds, pendEvals, solveCycles);
     if (lane == 0) {
         if (toSlow) list[atomicAdd(list_count, 1)] = pid;
         else {
@@ -656,6 +665,217 @@ __global__ void k_grid_size_scatter(int firstPair, const int* __restrict__ list,
     const int pid = list[t];
     if (qstatus[t] == 0) recs.max_arrv[(size_t)firstPair + pid] = metrics[t].throughput / 1000.0f;
     status[pid] = qstatus[t] == 0 ? 1 : 2;
+}
+
+// ---------------------------------------------------------------------------------------
+// wva_analyze_scenarios: Server.Calculate of every shard pair under L load scenarios, scenario l replacing each server's
+// arrival rate by rates[l*S + s].  Every input of QueueAnalyzer.Size is independent of the arrival rate
+// (allocation.go:77-131), so a pair runs Size once; per scenario only the nil / zero-load branches (:50, :73-75), the
+// replica count, the cost and the trailing Analyze(totalRate / replicas) (:133-160) remain.  The records of scenario l
+// are the S*A records at offset l*S*A of one record set.
+//   k_scen_pairs_warp   one warp per pair: Size through warp_pair_size<PAIR_SCEN>, then the scenarios 32 at a time,
+//                       lane = scenario, one warp_solve for all lanes; pairs it cannot finish are listed;
+//   k_scen_gather -> k_queue_size -> k_scen_rows -> k_queue_analyze -> k_scen_scatter
+//                       the listed pairs (every pair on the thread path): Size and the per-scenario Analyze through the
+//                       batched analyzer kernels (materialised-p[] re-runs included), records composed by the scatter.
+// ---------------------------------------------------------------------------------------
+
+// the nil checks of Server.Calculate + CreateAllocation that do not read the arrival rate (server.go:70-82,
+// allocation.go:41-70 without :50)
+__device__ __forceinline__ bool scen_pair_usable(const DevSystem& sys, int s, int a) {
+    if (!is_candidate_accel(sys, s, a)) return false;
+    if (sys.srv_in_tokens[s] < 0 || sys.srv_out_tokens[s] < 0) return false;
+    const int m = sys.srv_model[s];
+    if (m < 0 || m >= sys.M) return false;
+    if (!sys.perf_valid[(size_t)m * sys.A + a]) return false;
+    return sys.srv_target_valid[s] != 0;
+}
+
+// does server s see a positive rate in any scenario (else its pairs need no Size)
+__device__ __forceinline__ bool scen_any_positive(const float* __restrict__ rates, int L, int S, int s, int from, int step) {
+    bool any = false;
+    for (int l = from; l < L; l += step) any |= rates[(size_t)l * S + s] > 0.0f;
+    return any;
+}
+
+// N of CreateAllocation (allocation.go:77-87)
+__device__ __forceinline__ long long scen_batch(const DevSystem& sys, int s, int a) {
+    if (sys.srv_max_batch[s] > 0) return sys.srv_max_batch[s];
+    const size_t pi = (size_t)sys.srv_model[s] * sys.A + a;
+    const long long N = go_divi(go_muli(sys.perf_max_batch[pi], sys.perf_at_tokens[pi]), (long long)sys.srv_out_tokens[s]);
+    return N < 1 ? 1 : N;
+}
+
+#define WVA_SCEN_NIL  0    // CreateAllocation returns nil
+#define WVA_SCEN_ZERO 1    // zeroLoadAllocation: `rec` is the allocation
+#define WVA_SCEN_RATE 2    // Analyze(rate2) decides; numReplicas and cost are set
+// One scenario of a usable pair up to its trailing Analyze (allocation.go:50, :73-75, :133-147).  sized / rateStar:
+// the pair's Size succeeded with metrics.Throughput rateStar.
+__device__ __forceinline__ int scen_step(const DevSystem& sys, int s, int a, float r, bool sized, float rateStar,
+                                         long long& numReplicas, float& cost, float& rate2, AllocRec& rec) {
+    if (r < 0.0f) return WVA_SCEN_NIL;
+    const long long Kt = sys.srv_out_tokens[s];
+    if (r == 0.0f || Kt == 0) { rec = zero_load_allocation(sys, s, a); return WVA_SCEN_ZERO; }
+    if (!sized) return WVA_SCEN_NIL;
+    const float tTPS = sys.srv_slo_tps[s];
+    float totalRate;
+    if (tTPS == 0.0f) totalRate = r / 60.0f;
+    else totalRate = tTPS / (float)Kt;
+    numReplicas = go_f64_to_int(ceil((double)totalRate / (double)rateStar));
+    if (numReplicas < (long long)sys.srv_min_replicas[s]) numReplicas = sys.srv_min_replicas[s];
+    cost = sys.acc_cost[a] * (float)go_muli(num_instances(sys, sys.srv_model[s], a), numReplicas);
+    rate2 = totalRate / (float)numReplicas;
+    return WVA_SCEN_RATE;
+}
+
+// the allocation once Analyze(rate2) returned m2 (allocation.go:150-160)
+__device__ __forceinline__ AllocRec scen_alloc(int a, long long N, long long numReplicas, float cost, float rateStar,
+                                               const wva_metrics& m2) {
+    AllocRec rec;
+    rec.acc = a; rec.numReplicas = numReplicas; rec.batchSize = N;
+    rec.cost = cost; rec.itl = m2.avg_token_time;
+    rec.ttft = m2.avg_wait_time + m2.avg_prefill_time;
+    rec.rho = m2.rho; rec.maxArrv = rateStar / 1000.0f;
+    rec.value = cost;
+    return rec;
+}
+
+// record i of the scenario set: the allocation with its transition penalty (server.go:62-64), or nil
+__device__ __forceinline__ void scen_store(const DevSystem& sys, int s, const DevAllocs& recs, unsigned char* feasible, size_t i,
+                                           bool ok, AllocRec rec) {
+    if (ok) rec.value = transition_penalty(sys.srv_cur_acc[s], sys.srv_cur_replicas[s], sys.srv_cur_cost[s], rec.acc,
+                                           rec.numReplicas, rec.cost);
+    else rec = empty_alloc();
+    store_alloc(recs, i, rec);
+    feasible[i] = ok ? 1 : 0;
+}
+
+__global__ void __launch_bounds__(WVA_PAIRS_WARP_THREADS)
+k_scen_pairs_warp(DevSystem sys, int s0, int nPairs, int L, const float* __restrict__ rates, DevAllocs recs,
+                  unsigned char* __restrict__ feasible, int* list, int* list_count, int smemEntriesPerWarp) {
+    extern __shared__ __align__(16) unsigned char scen_smem[];
+    const int pid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;      // warp-uniform
+    const int lane = threadIdx.x & 31;
+    if (pid >= nPairs) return;
+    const int S = sys.S;
+    const int s = s0 + pid / sys.A, a = pid % sys.A;
+    const size_t gi = (size_t)s * sys.A + a, SA = (size_t)S * sys.A;
+    const bool usable = scen_pair_usable(sys, s, a);
+    const bool anyPos = __any_sync(0xffffffffu, scen_any_positive(rates, L, S, s, lane, 32));
+    PairModel pm;
+    pm.rateStar = 0.0f;
+    bool sized = false, toSlow = false;
+    unsigned long long steps = 0;
+    if (usable && anyPos && sys.srv_out_tokens[s] != 0) {
+        int activeRounds = 0, totalRounds = 0, pendEvals = 0;
+        long long solveCycles = 0;
+        AllocRec rec = empty_alloc();
+        warp_pair_size<PAIR_SCEN>(sys, s, a, pid, lane, 0, nullptr, nullptr, scen_smem, smemEntriesPerWarp, nullptr, 0, nullptr,
+                                  rec, sized, toSlow, steps, activeRounds, totalRounds, pendEvals, solveCycles, &pm);
+    }
+    for (int base = 0; base < L && !toSlow; base += 32) {
+        const int l = base + lane;
+        const bool active = l < L;
+        AllocRec rec = empty_alloc();
+        long long reps = 0;
+        float cost = 0.0f, rate2 = 0.0f;
+        const int kind = (active && usable) ? scen_step(sys, s, a, rates[(size_t)l * S + s], sized, pm.rateStar, reps, cost, rate2, rec)
+                                            : WVA_SCEN_NIL;
+        bool ok = kind == WVA_SCEN_ZERO;
+        // Analyze's range checks (queueanalyzer.go:135-143), as k_pairs_warp
+        const bool need = kind == WVA_SCEN_RATE && !(rate2 <= 0.0f || rate2 > pm.wp.rateMax);
+        // lanes with the same rate2 share one evaluation: every positive scenario of a TPS-target server has the same
+        const unsigned long long key = need ? (unsigned long long)__float_as_uint(rate2) : (0x100000000ull | (unsigned)lane);
+        const int leader = __ffs(__match_any_sync(0xffffffffu, key)) - 1;
+        const bool eval = need && leader == lane;
+        if (__any_sync(0xffffffffu, eval)) {
+            SolveStats st;
+            st.rho = st.avgNumInServers = st.avgNumInSystem = st.throughput = st.avgRespTime = st.avgServTime = st.avgWaitTime = 0.0f;
+            bool v = false, uu;
+            const bool solved = warp_solve(pm.wp, eval, rate2 / 1000.0f, st, steps, v, false, uu);
+            if (__any_sync(0xffffffffu, eval && !solved)) { toSlow = true; break; }
+            st = shfl_stats(st, leader);
+            v = __shfl_sync(0xffffffffu, (int)v, leader);
+            if (need && v) {
+                wva_metrics m2; metrics_from(pm.wp, st, m2);
+                rec = scen_alloc(a, pm.wp.N, reps, cost, pm.rateStar, m2);
+                ok = true;
+            }
+        }
+        if (active) scen_store(sys, s, recs, feasible, (size_t)l * SA + gi, ok, rec);
+    }
+    if (toSlow && lane == 0) list[atomicAdd(list_count, 1)] = pid;
+}
+
+// k_queue_size inputs of the listed pairs (list == nullptr: every shard pair): CreateAllocation's configuration
+// {N, 10 N, alpha, beta, gamma, delta, in, out} and the server's {TTFT, ITL, TPS}.  A pair that needs no Size (not
+// usable, no output tokens, no positive scenario rate) gets N = 0: k_queue_size then fails its configuration check
+// without running anything.
+__global__ void k_scen_gather(DevSystem sys, int s0, const int* __restrict__ list, int n, int L, const float* __restrict__ rates,
+                              wva_queue_config* __restrict__ cfg, float* __restrict__ target) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    const int pid = list ? list[t] : t;
+    const int s = s0 + pid / sys.A, a = pid % sys.A;
+    wva_queue_config c;
+    c.max_batch_size = 0; c.max_queue_size = 0;
+    c.alpha = c.beta = c.gamma = c.delta = 0.0f;
+    c.avg_input_tokens = sys.srv_in_tokens[s]; c.avg_output_tokens = sys.srv_out_tokens[s];
+    if (scen_pair_usable(sys, s, a) && sys.srv_out_tokens[s] != 0 && scen_any_positive(rates, L, sys.S, s, 0, 1)) {
+        const size_t pi = (size_t)sys.srv_model[s] * sys.A + a;
+        const long long N = scen_batch(sys, s, a);
+        c.max_batch_size = (int)N; c.max_queue_size = (int)go_muli(N, WVA_MAX_QUEUE_TO_BATCH_RATIO);
+        c.alpha = sys.perf_alpha[pi]; c.beta = sys.perf_beta[pi]; c.gamma = sys.perf_gamma[pi]; c.delta = sys.perf_delta[pi];
+    }
+    cfg[t] = c;
+    target[3 * t] = sys.srv_slo_ttft[s]; target[3 * t + 1] = sys.srv_slo_itl[s]; target[3 * t + 2] = sys.srv_slo_tps[s];
+}
+
+// k_queue_analyze inputs, one row per (listed pair t, scenario l) at t*L + l: the pair's configuration and rate2 where
+// the scenario reaches the trailing Analyze, else N = 0 (configuration check fails, nothing runs)
+__global__ void k_scen_rows(DevSystem sys, int s0, const int* __restrict__ list, int n, int L, const float* __restrict__ rates,
+                            const wva_queue_config* __restrict__ cfg, const wva_metrics* __restrict__ qmetrics,
+                            const unsigned char* __restrict__ qstatus, wva_queue_config* __restrict__ rcfg, float* __restrict__ rrate) {
+    const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= (size_t)n * L) return;
+    const int t = (int)(idx / L), l = (int)(idx % L);
+    const int pid = list ? list[t] : t;
+    const int s = s0 + pid / sys.A, a = pid % sys.A;
+    AllocRec rec;
+    long long reps = 0;
+    float cost = 0.0f, rate2 = 0.0f;
+    const int kind = scen_pair_usable(sys, s, a)
+                         ? scen_step(sys, s, a, rates[(size_t)l * sys.S + s], qstatus[t] == 0, qmetrics[t].throughput, reps, cost, rate2, rec)
+                         : WVA_SCEN_NIL;
+    wva_queue_config c = cfg[t];
+    if (kind != WVA_SCEN_RATE) c.max_batch_size = 0;
+    rcfg[idx] = c;
+    rrate[idx] = kind == WVA_SCEN_RATE ? rate2 : 0.0f;
+}
+
+// the records of the listed pairs from their Size (qmetrics / qstatus per pair) and Analyze rows (ametrics / astatus)
+__global__ void k_scen_scatter(DevSystem sys, int s0, const int* __restrict__ list, int n, int L, const float* __restrict__ rates,
+                               const wva_queue_config* __restrict__ cfg, const wva_metrics* __restrict__ qmetrics,
+                               const unsigned char* __restrict__ qstatus, const wva_metrics* __restrict__ ametrics,
+                               const unsigned char* __restrict__ astatus, DevAllocs recs, unsigned char* __restrict__ feasible) {
+    const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= (size_t)n * L) return;
+    const int t = (int)(idx / L), l = (int)(idx % L);
+    const int pid = list ? list[t] : t;
+    const int s = s0 + pid / sys.A, a = pid % sys.A;
+    AllocRec rec = empty_alloc();
+    long long reps = 0;
+    float cost = 0.0f, rate2 = 0.0f;
+    const float rateStar = qmetrics[t].throughput;
+    const int kind = scen_pair_usable(sys, s, a)
+                         ? scen_step(sys, s, a, rates[(size_t)l * sys.S + s], qstatus[t] == 0, rateStar, reps, cost, rate2, rec)
+                         : WVA_SCEN_NIL;
+    bool ok = kind == WVA_SCEN_ZERO;
+    if (kind == WVA_SCEN_RATE && astatus[idx] == WVA_CAND_OK) {
+        rec = scen_alloc(a, cfg[t].max_batch_size, reps, cost, rateStar, ametrics[idx]);
+        ok = true;
+    }
+    scen_store(sys, s, recs, feasible, (size_t)l * sys.S * sys.A + (size_t)s * sys.A + a, ok, rec);
 }
 
 // N per pair (0 = no queueing work) — used to order pairs by chain length and to size scratch.
@@ -1975,12 +2195,26 @@ k_queue_size(int n, const wva_queue_config* __restrict__ cfg, const float* __res
 // Optimize
 // ---------------------------------------------------------------------------------------
 
+__device__ __forceinline__ DevAllocs allocs_at(const DevAllocs& o, size_t off) {
+    DevAllocs r;
+    r.acc = o.acc + off; r.num_replicas = o.num_replicas + off; r.batch_size = o.batch_size + off;
+    r.cost = o.cost + off; r.value = o.value + off; r.itl = o.itl + off; r.ttft = o.ttft + off; r.rho = o.rho + off;
+    r.max_arrv = o.max_arrv + off;
+    return r;
+}
+
 // SolveUnlimited, solver.go:63-79: per server argmin of value with strict '<' from MaxFloat32,
 // candidates visited in ascending accelerator index (canonical order for Go's random map order).
+// blockIdx.y selects a record set (wva_analyze_scenarios: one per scenario) at pairStride records / flags, and its
+// solution at chosenStride; a single set runs with gridDim.y = 1.
 __global__ void k_solve_unlimited(DevSystem sys, int s0, int ns, DevAllocs pairs, const unsigned char* __restrict__ feasible,
-                                  int* __restrict__ chosen_acc, DevAllocs chosen) {
+                                  int* __restrict__ chosen_acc, DevAllocs chosen, size_t pairStride, size_t chosenStride) {
     int sl = blockIdx.x * blockDim.x + threadIdx.x;
     if (sl >= ns) return;
+    if (blockIdx.y) {
+        pairs = allocs_at(pairs, blockIdx.y * pairStride); feasible += blockIdx.y * pairStride;
+        chosen = allocs_at(chosen, blockIdx.y * chosenStride); chosen_acc += blockIdx.y * chosenStride;
+    }
     int s = s0 + sl;
     float minVal = 3.40282346638528859811704183484516925e+38f;
     int minKey = -1;
@@ -1999,12 +2233,17 @@ __global__ void k_solve_unlimited(DevSystem sys, int s0, int ns, DevAllocs pairs
 // servers' contributions in shared memory in parallel, then warp 0 adds them in order (a server
 // of another type contributes +0, which leaves a float32 sum that started at +0 unchanged).
 // The int64 unit counts wrap and are associative: plain tree reduction.
-// totals = { long long count[T]; float cost[T] }.
+// totals = { long long count[T]; float cost[T] }.  blockIdx.y selects a solution (wva_analyze_scenarios: one per
+// scenario) at chosenStride servers, whose totals go to count / cost + blockIdx.y * T.
 __global__ void __launch_bounds__(1024) k_totals(DevSystem sys, int s0, int ns, const int* __restrict__ chosen_acc, DevAllocs chosen,
-                                                 long long* __restrict__ count, float* __restrict__ cost) {
+                                                 long long* __restrict__ count, float* __restrict__ cost, size_t chosenStride) {
     __shared__ float vals[1024];
     __shared__ long long part[32];
     const int t = blockIdx.x;
+    if (blockIdx.y) {
+        chosen = allocs_at(chosen, blockIdx.y * chosenStride); chosen_acc += blockIdx.y * chosenStride;
+        count += (size_t)blockIdx.y * sys.T; cost += (size_t)blockIdx.y * sys.T;
+    }
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     long long c = 0; float k = 0.0f;
     for (int base = 0; base < ns; base += 1024) {

@@ -6,8 +6,9 @@
  *     silently change the Go-side layout fails here;
  * (3) on a box with a B200: the *_arrays entry points (what go/internal/native calls -- no struct of
  *     pointers crosses the boundary) give the same bytes as the struct forms, for the pair records and for
- *     the sweep's per-pair winners (wva_grid_pairs_fetch, wva_solve_grid); wva_grid_pairs_size flags every
- *     sweep record and nothing else.
+ *     the sweep's per-pair winners (wva_grid_pairs_fetch, wva_solve_grid) and for the load scenarios
+ *     (wva_analyze_scenarios, wva_scenario_pairs_fetch); wva_grid_pairs_size flags every sweep record and
+ *     nothing else.
  * Exit code 0 = ok (prints "no device" and stops after (2) when CUDA is unavailable). */
 #include <stddef.h>
 #include <stdio.h>
@@ -110,6 +111,23 @@ int main(void) {
     CHECK(wva_analyze_grid_device(ctx, 8, 32, 0) == WVA_OK);
     CHECK(wva_solve_grid(ctx, &spec, key2, &c2) == WVA_ESTATE);                 /* a sweep with the option off */
     CHECK(wva_grid_pairs_size(ctx, gst) == WVA_ESTATE);
+    /* load scenarios (the image's rates, none, twice the image's): arrays forms against struct forms */
+    enum { L = 3 };
+    float lr[L * S];
+    for (int i = 0; i < S; ++i) { lr[i] = sar[i]; lr[S + i] = 0.0f; lr[2 * S + i] = 2.0f * sar[i]; }
+    int32_t lkey1[L * S], lacc1[L * S], lkey2[L * S], lacc2[L * S]; int64_t lrep1[L * S], lbat1[L * S], lrep2[L * S], lbat2[L * S];
+    float lf1[6][L * S], lf2[6][L * S]; int64_t lcnt1[L * T], lcnt2[L * T]; float lcst1[L * T], lcst2[L * T];
+    CHECK(wva_analyze_scenarios_arrays(ctx, L, lr, lkey1, lacc1, lrep1, lbat1, lf1[0], lf1[1], lf1[2], lf1[3], lf1[4], lf1[5], lcnt1, lcst1) == WVA_OK);
+    CHECK(wva_scenario_pairs_fetch_arrays(ctx, 2, gacc1, grep1, gbat1, gf1[0], gf1[1], gf1[2], gf1[3], gf1[4], gf1[5], gfe1) == WVA_OK);
+    wva_alloc_soa l2 = {lacc2, lrep2, lbat2, lf2[0], lf2[1], lf2[2], lf2[3], lf2[4], lf2[5]};
+    CHECK(wva_analyze_scenarios(ctx, L, lr, lkey2, &l2, lcnt2, lcst2) == WVA_OK);
+    CHECK(wva_scenario_pairs_fetch(ctx, 2, &g2, gfe2) == WVA_OK);
+    CHECK(!memcmp(lkey1, lkey2, sizeof lkey1) && !memcmp(lacc1, lacc2, sizeof lacc1) && !memcmp(lrep1, lrep2, sizeof lrep1));
+    CHECK(!memcmp(lbat1, lbat2, sizeof lbat1) && !memcmp(lf1, lf2, sizeof lf1) && !memcmp(lcnt1, lcnt2, sizeof lcnt1) && !memcmp(lcst1, lcst2, sizeof lcst1));
+    CHECK(!memcmp(gacc1, gacc2, sizeof gacc1) && !memcmp(grep1, grep2, sizeof grep1) && !memcmp(gbat1, gbat2, sizeof gbat1));
+    CHECK(!memcmp(gf1, gf2, sizeof gf1) && !memcmp(gfe1, gfe2, sizeof gfe1));
+    CHECK(wva_analyze_scenarios(ctx, 0, lr, NULL, NULL, NULL, NULL) == WVA_EINVAL);
+    CHECK(wva_scenario_pairs_fetch(ctx, L, &g2, gfe2) == WVA_EINVAL);
     printf("cabi_test: ok (%d feasible pairs, %d feasible sweep pairs, type counts %lld %lld)\n", nfe, ngfe, (long long)cnt[0], (long long)cnt[1]);
     wva_ctx_destroy(ctx);
     return 0;
